@@ -92,6 +92,28 @@ class ClockSampler(object):
                 "samples": len(sm)}
 
 
+DUMP_SAMPLE = 1 << 21      # parameter entries written per module by --dump-outputs (8 MB of float32 each)
+
+
+def dump_outputs(out_dir, losses, modules):
+    """What the timed step hands back, as DIR/<name>.npy: loss_d and loss_g (float64), and the parameters the step
+    updated in place, flattened in named_parameters() order (float32) -- a fixed seeded sample of DUMP_SAMPLE
+    positions when a module has more, so that runs with the same arguments compare position for position.  The inputs
+    are the same from run to run; the outputs agree to a tolerance, not bit for bit, because the weight-gradient
+    kernels accumulate with float atomics."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in zip(("loss_d", "loss_g"), losses):
+        np.save(os.path.join(out_dir, name + ".npy"), np.array(float(v), dtype=np.float64))
+    for name, m in modules:
+        flat = torch.cat([p.detach().reshape(-1).float() for p in m.parameters()])
+        if flat.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(out_dir, name + "_params.npy"), flat.cpu().numpy())
+
+
 def train_params(gp_lambda, frame_sizes=(8, 16, 32, 64)):
     return SimpleNamespace(data_is_imgs=False, img_model=False, frame_sizes=list(frame_sizes), subsample_input=True,
                            discrim_steps=1, gen_steps=1, gp_lambda=gp_lambda, no_mean_discrim_loss=False,
@@ -273,10 +295,12 @@ def run_b200(args):
             return graphed(x, [t, l])
 
     res_evt = [torch.cuda.Event() for _ in range(3)]
+    last_out = {}
 
     def step_resident(i):
         x, t, l = dev[i % nb]
         out = run_step(x, t, l)
+        last_out["losses"] = out
         # keep the host two steps ahead at most (what the launch queue allows on one GPU anyway): with NCCL between the
         # graph replays an unbounded run-ahead measured 128 ms / step at two GPUs against 92 ms through the e2e loop
         res_evt[i % 3].record()
@@ -361,6 +385,8 @@ def run_b200(args):
     t_res = timed(step_resident, args.steps)
     launches = launches_per_step * args.steps
     clk = clocks.stop() if sample_clocks else None
+    if args.dump_outputs and rank == 0:                           # the legs below keep training the same modules
+        dump_outputs(args.dump_outputs, last_out["losses"], (("gen", gen), ("dis", dis)))
     timed(step_e2e, 3, begin=e2e_begin, end=e2e_end)               # e2e warm-up (staging slots, pinned pages)
     t_e2e = timed(step_e2e, args.steps, begin=e2e_begin, end=e2e_end)
 
@@ -527,6 +553,9 @@ def main():
     ap.add_argument("--lib_batches", type=int, nargs="+", default=[64, 256],
                     help="batches of the torch-eager cuDNN comparator (library_baseline / --impl torch_cuda)")
     ap.add_argument("--eager", action="store_true", help="no CUDA graphs: launch every kernel from Python")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's losses and a sample of the updated G / D "
+                         "parameters to DIR/<name>.npy (b200 arm)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -1,15 +1,12 @@
 """CPU: host-side pieces added around the kernels -- checkpoint compatibility with the reference (SURVEY 8f3), the
 position-pair identity behind the small-channel weight gradients, lagged loss logging, the prefetcher's CPU path."""
 import os
-import sys
 
 import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import build_product_models
-
-REF = "/root/reference"
+from helpers import build_product_models, golden
 
 
 def test_checkpoint_roundtrip_through_cond_gan(tmp_path):
@@ -32,33 +29,24 @@ def test_checkpoint_roundtrip_through_cond_gan(tmp_path):
         assert all(torch.equal(sa[k], sb[k]) for k in sa)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout is only present in the build container")
 def test_state_dicts_interchange_with_the_reference_modules():
-    """A reference-trained checkpoint loads into the product modules and vice versa (strict): same keys, same shapes
-    (models/tganv2_cond/{gen,discrim}.py, models/txt/basic.py)."""
-    # import the REFERENCE's txt2vid package in isolation from this repo's namespace package of the same name
-    stash = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "txt2vid" or k.startswith("txt2vid.")}
-    sys.path.insert(0, REF)
-    try:
-        from txt2vid.models.tganv2_cond.gen import MultiScaleGen as RefGen
-        from txt2vid.models.tganv2_cond.discrim import MultiScaleDiscrim as RefDis
-        from txt2vid.models.txt.basic import Seq2Seq as RefTxt
-        assert sys.modules["txt2vid.models.tganv2_cond.gen"].__file__.startswith(REF)
-    except ImportError as e:
-        pytest.skip("reference modules not importable here: %r" % (e,))
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "txt2vid" or k.startswith("txt2vid.")]:
-            del sys.modules[k]
-        sys.modules.update(stash)
-    txt, gen, dis = build_product_models(True, V=50, seed=3)
-    rgen, rdis, rtxt = RefGen(width=64, height=64, cond_dim=256), RefDis(cond_dim=256), RefTxt(vocab_size=50)
-    for prod, ref in ((gen, rgen), (dis, rdis), (txt, rtxt)):
-        ref.load_state_dict(prod.state_dict(), strict=True)            # product checkpoint -> reference
-        prod.load_state_dict(ref.state_dict(), strict=True)            # reference checkpoint -> product
-        sp, sr = prod.state_dict(), ref.state_dict()
-        assert list(sp) == list(sr)
-        assert all(sp[k].shape == sr[k].shape and torch.equal(sp[k].float(), sr[k].float()) for k in sp)
+    """A reference checkpoint's tensors line up with the product modules (models/tganv2_cond/{gen,discrim}.py,
+    models/txt/basic.py): every floating-point state_dict entry the reference's modules recorded in the golden fixture
+    (oracle/make_golden.py), with the same name, in the same order, with the same element count; and a product
+    checkpoint loads back strictly into fresh product modules."""
+    fx = golden("tganv2_cond_B8.json")
+    txt, gen, dis = build_product_models(True, V=fx["config"]["V"], seed=fx["config"]["seed"])
+    txt2, gen2, dis2 = build_product_models(True, V=fx["config"]["V"], seed=fx["config"]["seed"] + 1)
+    for part, prod, fresh in (("gen", gen, gen2), ("dis", dis, dis2), ("txt", txt, txt2)):
+        ref = fx["init"][part]
+        sp = prod.state_dict()
+        mine = [(k, v) for k, v in sp.items() if v.dtype.is_floating_point]
+        assert [k for k, _ in mine] == list(ref), part
+        assert all(v.numel() == ref[k]["n"] for k, v in mine), part
+        fresh.load_state_dict(sp, strict=True)
+        sf = fresh.state_dict()
+        assert list(sf) == list(sp)
+        assert all(sf[k].shape == sp[k].shape and torch.equal(sf[k], sp[k]) for k in sp)
 
 
 def test_position_pair_identity_of_small_channel_weight_gradients():
@@ -108,79 +96,42 @@ def test_prefetcher_cpu_path_and_deferred_preload():
         assert got == [(float(i), i, [4, 4]) for i in range(5)]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout is only present in the build container")
 def test_caption_pretraining_step_matches_the_reference(monkeypatch):
-    """SURVEY 8(f4): one optimisation step of train/txt.py:166-181 (encode -> teacher-forced decode -> cross entropy
-    -> Adam) on identical weights and sentences: same loss, same decoded symbols, same updated weights.  The product's
-    embedding / LSTM recurrence / GEMM kernels are replaced by their executable spec (tests/cpu_kernels.py, fp32
-    storage): this checks the host logic and the autograd formulas of text.py against the LIVE reference."""
+    """SURVEY 8(f4): one step of train/txt.py:166-181 (encode -> teacher-forced / greedy decode -> cross entropy) on
+    the weights and sentences of the fixture recorded from the reference (oracle/make_golden_caption_pretrain.py):
+    same loss, the same decoded symbols in both modes, every parameter's gradient within 1e-4 (norm and probe).  The
+    product's embedding / LSTM recurrence / GEMM kernels are replaced by their executable spec (tests/cpu_kernels.py,
+    fp32 storage): this checks the host logic and the autograd formulas of text.py against the reference."""
     import cpu_kernels
+    from test_round2_gpu import _golden_caption, _probe_index
     from txt2vid_b200 import ops
+    from txt2vid_b200.text import Seq2Seq
+    from txt2vid_b200.train_txt import pretrain_step
     monkeypatch.setattr(ops, "K", cpu_kernels)
     cpu_kernels.set_store_dtype(torch.float32)
     ops.PACKS.clear()
     try:
-        _caption_pretraining_body()
+        fx = _golden_caption()
+        torch.manual_seed(fx["seed"])
+        prod = Seq2Seq(vocab_size=fx["V"])
+        for n, p in prod.state_dict().items():
+            s, a = fx["weights"][n]
+            assert abs(float(p.double().sum()) - s) <= 1e-9 * max(1.0, a), n
+        sent = torch.tensor(fx["sent"], dtype=torch.long)
+        for mode, tf in (("teacher_force", True), ("greedy", False)):
+            want = fx["modes"][mode]
+            loss_p, sym_p = pretrain_step(prod, sent, fx["lengths"], None, teacher_force=tf)
+            assert abs(float(loss_p) - want["loss"]) <= 2e-6 * abs(want["loss"]), (mode, float(loss_p), want["loss"])
+            assert sym_p.tolist() == want["symbols"], mode
+            for n, p in prod.named_parameters():
+                g, w = p.grad.detach().reshape(-1), want["grads"][n]
+                assert abs(float(g.double().norm()) - w["norm"]) <= 1e-4 * (w["norm"] + 1e-12), (mode, n)
+                probe = torch.tensor(w["probe"])
+                assert float((g[_probe_index(g.numel())] - probe).norm()) <= 1e-4 * (float(probe.norm()) + 1e-12), \
+                    (mode, n)
     finally:
         cpu_kernels.set_store_dtype(torch.bfloat16)
         ops.PACKS.clear()
-
-
-def _caption_pretraining_body():
-    stash = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "txt2vid" or k.startswith("txt2vid.")}
-    sys.path.insert(0, REF)
-    try:
-        from txt2vid.models.txt.basic import Seq2Seq as RefTxt
-        assert sys.modules["txt2vid.models.txt.basic"].__file__.startswith(REF)
-    except ImportError as e:
-        pytest.skip("reference modules not importable here: %r" % (e,))
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "txt2vid" or k.startswith("txt2vid.")]:
-            del sys.modules[k]
-        sys.modules.update(stash)
-    import contextlib, io
-    from torch.nn.utils.rnn import pack_padded_sequence, pad_packed_sequence
-    from txt2vid_b200.text import Seq2Seq
-    from txt2vid_b200.train_txt import collate_fn, pretrain_step
-    V = 40
-    torch.manual_seed(5)
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref = RefTxt(vocab_size=V)
-    prod = Seq2Seq(vocab_size=V)
-    prod.load_state_dict(ref.state_dict(), strict=True)
-    g = torch.Generator().manual_seed(1)
-    sents = []
-    for L in (9, 7, 7, 4):
-        s = torch.randint(4, V, (L,), generator=g).float()
-        s[0], s[-1] = 1, 2
-        sents.append(s)
-    sent, lengths = collate_fn(list(sents))
-    for tf in (True, False):
-        opt_r = torch.optim.Adam(ref.parameters(), lr=1e-3)
-        opt_p = torch.optim.Adam(prod.parameters(), lr=1e-3)
-        # the reference's loop body, verbatim order (train/txt.py:166-181)
-        ref.zero_grad()
-        _, hid, _ = ref.encode(sent, lengths=lengths)
-        targets, _ = pad_packed_sequence(pack_padded_sequence(sent, lengths, batch_first=True), batch_first=True,
-                                         total_length=lengths[0])
-        dec, sym = ref.decode(true_inputs=sent, initial_hidden=hid, max_seq_len=lengths[0], teacher_force=tf)
-        loss_r = torch.nn.CrossEntropyLoss()(dec.permute(0, 2, 1), targets)
-        loss_r.backward()
-        loss_p, sym_p = pretrain_step(prod, sent, lengths, None, teacher_force=tf)
-        assert abs(float(loss_p) - float(loss_r)) <= 2e-6 * abs(float(loss_r)), (float(loss_p), float(loss_r))
-        assert torch.equal(sym_p, sym)
-        # gradients of every parameter (the kernels sum in a different order than ATen: 1e-4 relative; Adam's first
-        # step is sign-like, so the updated weights themselves are compared on the tensors' scale)
-        for (n, a), (_, b) in zip(prod.named_parameters(), ref.named_parameters()):
-            assert a.grad is not None and b.grad is not None, n
-            err = float((a.grad - b.grad).norm() / (b.grad.norm() + 1e-12))
-            assert err < 1e-4, (n, err)
-        opt_r.step()
-        opt_p.step()
-        for (n, a), (_, b) in zip(prod.state_dict().items(), ref.state_dict().items()):
-            assert float((a - b).abs().max()) <= 2.1e-3, n          # at most one sign flip of a 1e-3 Adam step
-        prod.load_state_dict(ref.state_dict(), strict=True)
 
 
 def test_caption_pretraining_golden_fixture_through_the_executable_spec(monkeypatch):
@@ -243,26 +194,3 @@ def test_trainer_test_writes_the_reference_sample_files(tmp_path, emulated_fp32)
     im = Image.open(os.path.join(params.out_samples, "64x64_0_0.jpg"))
     assert im.size == (16 * 64 + 17 * 2, 2 * 64 + 3 * 2)                             # nrow = 16 frames, 2 clips, padding 2
 
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout is only present in the build container")
-def test_pickled_reference_sentence_model_loads_into_the_product(tmp_path, emulated_fp32):
-    """SURVEY 8(f3): train/txt.py:190-191 saves the WHOLE caption model with torch.save(model) and train/gan.py:38-42
-    loads that pickle (`--sent_weights`).  A pickle written by the live reference (subprocess with /root/reference on
-    the path) must unpickle under this repo's `txt2vid` namespace into the product's Seq2Seq and encode identically."""
-    import subprocess
-    path, out = str(tmp_path / "sent.pth"), str(tmp_path / "ref_out.pt")
-    code = ("import sys, torch; sys.path.insert(0, %r); torch.manual_seed(7)\n"
-            "from txt2vid.models.txt.basic import Seq2Seq\n"
-            "m = Seq2Seq(vocab_size=40)\n"
-            "tok = torch.tensor([[1, 5, 6, 7, 2], [1, 9, 2, 0, 0]]); lens = [5, 3]\n"
-            "o, (h, c), hn = m.encode(tok, lens)\n"
-            "torch.save(m, %r); torch.save({'tok': tok, 'lens': lens, 'out': o, 'h': h, 'c': c, 'hn': hn}, %r)\n"
-            % (REF, path, out))
-    subprocess.check_call([sys.executable, "-c", code], cwd=str(tmp_path))
-    import txt2vid_b200.text as T
-    m = torch.load(path, weights_only=False)
-    assert type(m) is T.Seq2Seq and type(m.encoder) is T.RecurrentModel
-    ref = torch.load(out)
-    o, (h, c), hn = m.encode(ref["tok"], ref["lens"])
-    for a, b in ((o, ref["out"]), (h, ref["h"]), (c, ref["c"]), (hn, ref["hn"])):
-        assert a.shape == b.shape and float((a.float() - b).abs().max()) < 1e-5
