@@ -45,8 +45,6 @@ extern "C" {
 #define T2V_EPI_RELU_MASK 4u  /* the `residual` pointer is a ReLU reference r (bf16 CL, output-shaped): instead of
                                * adding it, zero the output where r <= 0 -- the backward of the ReLU that produced the
                                * convolution's input, fused into the data-gradient epilogue (layers.py:230-232) */
-#define T2V_EPI_RES_F32 8u    /* the `residual` / ReLU-reference pointer is fp32 CL (fp32 activation storage, generic
-                               * tcgen05 kernel only) */
 #define T2V_EPI_IN_F32 16u    /* fp32 PARITY mode: x / residual are fp32 CL and w is fp32 [Cout][taps][Cin]; the
                                * convolution runs as exact fp32 FMAs on the CUDA cores (the reference's numerics; the
                                * tensor pipe's truncating fp32 accumulator cannot reach 1e-6 on K ~ 1e4), y fp32 */
@@ -329,18 +327,14 @@ int t2v_adam_step(int32_t count, float* const* host_params, const float* const* 
 /* gradient bucket pack / unpack for the data-parallel all-reduce (fp32, memory order): dst[i][:] = src[i][:]  */
 int t2v_multi_copy(int32_t count, const float* const* host_src, float* const* host_dst, const int64_t* host_sizes,
                    void* stream);
-/* Bulk copy by `ctas` resident CTAs with streaming loads / stores; src may be PINNED host memory (UVA): the input
- * batch of data/__init__.py:131-156's prefetcher without the copy engine.  nbytes a multiple of 16.            */
-int t2v_stream_copy(const void* src, void* dst, int64_t nbytes, int32_t ctas, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * fp32 ACTIVATION STORAGE (the "fp32 parity mode": BASELINE north_star, 1e-3 relative on losses and gradients).
  * Every entry point above whose activations are bf16 CL has a twin with the suffix _f32 and the SAME signature
  * in which those tensors are fp32 CL (same kernels instantiated for float storage; arithmetic is fp32 in both).
- * The tcgen05 engine keeps its bf16 tensor pipe: fp32 activations are split into bf16 hi + lo parts
- * (t2v_split_bf16x3), weights likewise, and hi*hi + lo*hi + hi*lo is accumulated in fp32 by the SAME kernels along a
- * 3x longer K (fprop / dgrad: channel-concatenated operands, T2V_EPI_OUT_F32 | T2V_EPI_RES_F32) or 3x more
- * positions (wgrad): ~2^-17 relative error per product.                                                         */
+ * Convolutions on fp32 storage bypass the bf16 tensor pipe and run as exact fp32 FMAs on the CUDA cores:
+ * t2v_conv_fprop / t2v_conv_dgrad with T2V_EPI_IN_F32, t2v_conv_wgrad with T2V_ALGO_SIMT_F32, and the
+ * t2v_gconv_*_f32 entry points below.                                                                          */
 int t2v_relu_fwd_f32(const void* x, void* y, int64_t n, void* stream);
 int t2v_relu_bwd_f32(const void* dy, const void* ref, void* dx, int64_t n, void* stream);
 int t2v_leaky_relu_fwd_f32(const void* x, void* y, int64_t n, float slope, void* stream);
@@ -383,15 +377,6 @@ int t2v_gconv_dgrad_f32(const t2v_gconv_geom* g, const void* dy, const void* w, 
                         int32_t out_f32, void* stream);
 int t2v_gconv_wgrad_f32(const t2v_gconv_geom* g, const void* dy, const void* x, float* dw, int32_t accumulate,
                         void* stream);
-/* x fp32 [rows][C] -> bf16 hi = bf16(x), lo = bf16(x - hi); layout 0: out [rows][3C] = [hi | lo | hi] (A operand of
- * fprop / dgrad; the weight pack is [hi | hi | lo] along K), 1: out [3 rows][C] = [hi ; lo ; hi] (dy of wgrad),
- * 2: out [3 rows][C] = [hi ; hi ; lo] (x of wgrad).  C a multiple of 4.                                        */
-int t2v_split_bf16x3(const float* x, void* out, int64_t rows, int32_t C, int32_t layout, void* stream);
-/* general form: terms = 3 as above; terms = 6 splits x = a + b + c (24 bits = fp32 operands) and lays out the six
- * products a a' + b a' + a b' + c a' + a c' + b b': layouts 0 / 1 = [a | b | a | c | a | b] (activations), layout 2
- * and the weight packs = [a | a | b | a | c | b].  This is the fp32 parity mode's default (error <= 2^-23 per
- * product: ReLU masks of the fp32 oracle are reproduced, which a 2^-17 split does not guarantee).               */
-int t2v_split_bf16(const float* x, void* out, int64_t rows, int32_t C, int32_t layout, int32_t terms, void* stream);
 
 /* scale / add / dot on CL activations (bf16; _f32 twins): the non-local block's gamma * o + x
  * (models/layers.py:36,68) with its gradients, and the gradient penalty's sum ||g||^2 (gan/losses.py:180-186).

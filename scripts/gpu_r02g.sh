@@ -5,4 +5,3 @@ F='Warn\|Consider\|run_backward'
 timeout 1500 python -m pytest tests/test_iteration_gpu.py tests/test_round2_gpu.py tests/test_families.py tests/test_nrank_parity.py -m gpu -q -s --tb=short -p no:cacheprovider -k "fp32 or nrank or two_rank" 2>&1 | grep -v "$F" > gpurun_out/pytest_g.log
 grep -n "passed\|failed" gpurun_out/pytest_g.log | tail -3
 grep -n "^FAILED\|deviations\|fp32 mode\|2-rank\|Error" gpurun_out/pytest_g.log | cut -c1-700
-T2V_FP32_ENGINE=ffma timeout 300 python scripts/debug_fp32_conv.py 2>&1 | grep -v "$F" | cut -c1-200

@@ -1,5 +1,5 @@
 """Times the conv engine (fprop + wgrad, CUDA events, 20 launches after 3 warm-ups) on the TGANv2 shapes that
-carry the step at batch 1024 / GPU.  Usage: python scripts/perf_shapes.py [tag]  (env knobs select variants)."""
+carry the step at batch 1024 / GPU.  Usage: python scripts/perf_shapes.py [tag]  (the tag labels the output)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -32,6 +32,23 @@ def test_no_cpu_fallback():
                      k=(1, 1, 1))
 
 
+def test_environment_reads_are_diagnostics_and_launcher_variables_only():
+    """The product reads no environment variable that selects a code path or a tuning value: what runs depends on
+    the inputs and the code only.  Allowed are the diagnostics T2V_PROFILE_DUMP / T2V_DEBUG_LAUNCH (they print,
+    select nothing) and the launcher's rank variables."""
+    import glob
+    pkg = os.path.join(ROOT, "txt2vid_b200")
+    files = glob.glob(os.path.join(pkg, "**", "*.py"), recursive=True)
+    files += [p for p in glob.glob(os.path.join(pkg, "csrc", "*")) if p.endswith((".cu", ".cuh", ".inc", ".h"))]
+    files += glob.glob(os.path.join(ROOT, "include", "*.h"))
+    read = re.compile(r"""\b(?:environ\.get|getenv|env_int)\s*\(\s*["']([^"']+)["']|\benviron\s*\[\s*["']([^"']+)["']""")
+    names = set()
+    for path in files:
+        with open(path) as f:
+            names.update(a or b for a, b in read.findall(f.read()))
+    assert names == {"T2V_PROFILE_DUMP", "T2V_DEBUG_LAUNCH", "WORLD_SIZE", "RANK", "LOCAL_RANK"}, sorted(names)
+
+
 def test_vocab_and_collate_bit_exact():
     from txt2vid_b200.data import Vocab, build_vocab, collate_fn
     sents = ["digit 3 is left and right.", "Digit 7 is top and bottom", "a man is cooking."]

@@ -68,7 +68,7 @@ def _setup():
 
 
 # halo-resident fprop (Cin = Cout = 64): lines along h (H >= 16), lines along d (D >= 16, small H), 2-D maps,
-# ragged extents / partial tiles / dummy cluster tiles
+# ragged extents / partial tiles / dummy tiles
 HALO_FPROP_CASES = [
     (3, 2, 16, 16, 64, 64, (3, 3, 3)),
     (2, 5, 40, 24, 64, 64, (3, 3, 3)),

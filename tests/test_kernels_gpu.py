@@ -312,16 +312,3 @@ def test_data_prefetcher_uint8_frames_normalised_like_the_reference_transforms()
     x, y = pf.next()
     torch.cuda.synchronize()
     assert x.dtype == torch.float32 and torch.equal(x.cpu(), ref)
-
-
-def test_stream_copy_from_pinned_host_memory():
-    """t2v_stream_copy: bulk copy by a few resident CTAs, source in pinned host memory (UVA) or on the device."""
-    g = torch.Generator().manual_seed(5)
-    h = torch.rand(3, 1 << 20, generator=g).pin_memory()
-    d = torch.empty_like(h, device="cuda")
-    K().stream_copy(h, d, ctas=8)
-    torch.cuda.synchronize()
-    assert torch.equal(d.cpu(), h)
-    d2 = torch.empty_like(d)
-    K().stream_copy(d, d2, ctas=16)
-    assert torch.equal(d2, d)

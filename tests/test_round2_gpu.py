@@ -2,8 +2,8 @@
 (oracle/txt2vid_oracle.py: the restatement of the reference pinned to the live reference), and the fp32 storage mode
 of the whole engine at BASELINE north_star's fp32 bar (1e-3).
 
-  * fp32 storage twins of the HBM-bound kernels vs their executable spec, and the bf16x3 operand split of the tcgen05
-    engine vs F.conv3d in fp32 (TF32 off);
+  * fp32 storage twins of the HBM-bound kernels vs their executable spec, and the fp32 convolution engine (exact fp32
+    FMAs on the CUDA cores) vs F.conv3d in fp64;
   * non-local block (Attention3d with gamma != 0) forward, backward AND double backward vs oracle attention3d;
   * caption encoder (Embedding + 4-layer length-masked Bi-LSTM) forward / backward vs oracle seq2seq_encode;
   * discriminator heads + fused relativistic loss vs the oracle's per-level composition;
@@ -86,17 +86,17 @@ def test_fp32_storage_kernels_match_spec(precision):
     assert torch.equal(K().f32_pad_cl(sl, 32, dt)[..., :20].float(), sl.to(dt).float())
 
 
-@pytest.mark.parametrize("engine,tol", [("ffma", 3e-6), ("tc", 5e-5)])
+@pytest.mark.parametrize("epilogue", ["residual", "relu"])
 @pytest.mark.parametrize("geom", [((4, 1, 8, 8), 64, 64, (1, 3, 3)), ((2, 4, 4, 4), 128, 64, (3, 3, 3)),
                                   ((16, 1, 1, 1), 256, 512, (1, 1, 1)), ((2, 2, 8, 8), 16, 32, (3, 3, 3)),
                                   ((3, 1, 4, 4), 1024, 256, (1, 3, 3))])
-def test_conv_engine_fp32_mode(geom, engine, tol, monkeypatch):
-    """The two convolution engines of the fp32 storage mode against F.conv3d in fp32 (TF32 off): "ffma" (default: fp32
-    operands, exact fp32 FMAs on the CUDA cores, a few 1e-7 -- what the 1e-3 gradient bar needs) and "tc" (the tcgen05
-    engine on bf16 hi/lo part splits, a few 1e-5: the tensor pipe's accumulator truncates) -- fprop / dgrad / wgrad."""
+def test_conv_engine_fp32_mode(geom, epilogue):
+    """The convolution engine of the fp32 storage mode against F.conv3d in fp64 (TF32 off): fp32 operands, exact fp32
+    FMAs on the CUDA cores, a few 1e-7 -- what the 1e-3 gradient bar needs -- fprop (epilogue bias + residual, or
+    bias + ReLU) / dgrad / wgrad."""
     from txt2vid_b200 import ops
     (N, D, H, W), Cin, Cout, k = geom
-    monkeypatch.setattr(K(), "FP32_ENGINE", engine)
+    tol = 3e-6
     ops.set_precision("fp32")
     torch.backends.cudnn.allow_tf32 = False
     try:
@@ -108,8 +108,13 @@ def test_conv_engine_fp32_mode(geom, engine, tol, monkeypatch):
         w5 = w.view(Cout, k[0], k[1], k[2], Cin).permute(0, 4, 1, 2, 3).contiguous()
         pad = tuple(kk // 2 for kk in k)
         # fp64 reference (cuDNN's own fp32 kernels sit ~1e-6 from it on the K = 9216 case)
-        ref = F.conv3d(x.permute(0, 4, 1, 2, 3).double(), w5.double(), bias.double(), padding=pad).permute(0, 2, 3, 4, 1) + res
-        y = K().conv_fprop(x, K().pack_weight(w), bias, res, k)
+        ref = F.conv3d(x.permute(0, 4, 1, 2, 3).double(), w5.double(), bias.double(), padding=pad).permute(0, 2, 3, 4, 1)
+        if epilogue == "residual":
+            ref = ref + res
+            y = K().conv_fprop(x, K().pack_weight(w), bias, res, k)
+        else:
+            ref = ref.clamp_min(0)
+            y = K().conv_fprop(x, K().pack_weight(w), bias, None, k, relu=True)
         assert y.dtype == F32 and rel(y, ref) < tol, rel(y, ref)
         dy = torch.randn(N, D, H, W, Cout, device="cuda", generator=g)
         xr = x.permute(0, 4, 1, 2, 3).detach().double().requires_grad_(True)

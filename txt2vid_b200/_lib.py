@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libt2v_b200.so")
 
 T2V_OK = 0
 ALGO_AUTO, ALGO_TC, ALGO_SIMT, ALGO_TC_GENERIC, ALGO_SIMT_F32 = 0, 1, 2, 3, 4
-EPI_RELU, EPI_OUT_F32, EPI_RELU_MASK, EPI_RES_F32, EPI_IN_F32 = 1, 2, 4, 8, 16
+EPI_RELU, EPI_OUT_F32, EPI_RELU_MASK, EPI_IN_F32 = 1, 2, 4, 16
 
 
 class ConvGeom(ctypes.Structure):
@@ -76,7 +76,6 @@ SIGNATURES = {
     "t2v_stem_wgrad": [_P, _P, c_i32, _P, c_i64, c_i32, c_i32, c_i32, c_i32, _P],
     "t2v_rgb_to_cl": [_P, _P, _P, c_i64, c_i64, _P],
     "t2v_wgrad_fold_pairs": [_P, _P, c_i32, c_i32, c_i32, _P],
-    "t2v_stream_copy": [_P, _P, c_i64, c_i32, _P],
     "t2v_gconv_fprop": [ctypes.POINTER(GconvGeom), _P, _P, _P, _P, c_i32, _P],
     "t2v_gconv_dgrad": [ctypes.POINTER(GconvGeom), _P, _P, _P, _P, c_i32, _P],
     "t2v_gconv_wgrad": [ctypes.POINTER(GconvGeom), _P, _P, _P, c_i32, _P],
@@ -144,8 +143,6 @@ _TYPED = ["t2v_relu_fwd", "t2v_relu_bwd", "t2v_leaky_relu_fwd", "t2v_leaky_relu_
           "t2v_lstm_seq_bwd", "t2v_embedding_fwd", "t2v_embedding_bwd"]
 _F32P = ctypes.POINTER(ctypes.c_float)
 SIGNATURES.update({
-    "t2v_split_bf16x3": [_P, _P, c_i64, c_i32, c_i32, _P],
-    "t2v_split_bf16": [_P, _P, c_i64, c_i32, c_i32, c_i32, _P],
     "t2v_scale": [_P, _P, _P, c_i64, _P],
     "t2v_scale_add": [_P, _P, _P, _P, c_i64, _P],
     "t2v_dot": [_P, _P, _P, c_i64, _P],

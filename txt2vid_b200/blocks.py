@@ -10,8 +10,6 @@ never called.  Every block has two entry points:
   forward_cl(x)  channels-last bf16 tensors (N, D, H, W, C) -- used between blocks;
   forward(x)     the reference's signature (fp32, channel-first) -- converts at the boundary.
 """
-import os
-
 import torch
 import torch.nn as nn
 from torch.nn import Parameter as P
@@ -86,10 +84,9 @@ class Attention(nn.Module):
         # The 2-D block lives in the generator (never differentiated twice) and runs on the fused attention-core
         # kernels (t2v_attention_fwd/_bwd, parity-tested): the (P x P/4) attention matrix -- 1 GB fp32 per step at batch
         # 1024 -- never exists.  Measured on B200 (scripts/attn_probe.py, 1024 maps of 32x32): fused bwd 1.49 ms against
-        # 3.84 ms for the ATen composite's forward + backward.  T2V_FUSED_ATTENTION=0 selects the composite.  The
-        # discriminator's 3-D block is on the gradient-penalty path (double backward) and keeps the composite.
-        import os
-        self.fused_core = which_conv is nn.Conv2d and os.environ.get("T2V_FUSED_ATTENTION", "1") == "1"
+        # 3.84 ms for the ATen composite's forward + backward.  The discriminator's 3-D block is on the
+        # gradient-penalty path (double backward) and keeps the composite.
+        self.fused_core = which_conv is nn.Conv2d
 
     def forward_cl(self, x):
         return ops.nonlocal_block(x, self.theta.weight, self.phi.weight, self.g.weight, self.o.weight, self.gamma,
@@ -192,7 +189,7 @@ class DownBlock(nn.Module):
         c1 = self.main.identity_map[0]
         # both ReLU backward masks ride in the data-gradient epilogues of their (single) consumers
         h = ops.conv(ops.relu(x, later=True), m[1].weight, m[1].bias, relu=True, x_relu=True, relu_later=True)
-        if SKIP_FUSE and not ops.fp32_mode() and x.shape[-1] % 64 == 0 and h.shape[-1] % 64 == 0 \
+        if not ops.fp32_mode() and x.shape[-1] % 64 == 0 and h.shape[-1] % 64 == 0 \
                 and tuple(c1.weight.shape[2:]) == (1, 1, 1):
             # the 1^3 skip convolution is extra K of the second convolution's implicit GEMM
             h = ops.conv_skip(h, x, m[3].weight, m[3].bias, c1.weight, c1.bias, h_relu=True)
@@ -300,11 +297,6 @@ class ConvLSTM(nn.Module):
         return outputs, (outputs[-1], None)
 
 
-STEM_SD2 = os.environ.get("T2V_STEM_SD2", "1") == "1"
-STEM_DIRECT = os.environ.get("T2V_STEM_DIRECT", "1") == "1"
-SKIP_FUSE = os.environ.get("T2V_SKIP_FUSE", "1") == "1"
-
-
 class Resnet3D(nn.Module):
     """ResNet-3D discriminator trunk + unconditional / conditional heads (resnet3d.py:6-57)."""
 
@@ -332,7 +324,7 @@ class Resnet3D(nn.Module):
     def features(self, x):
         """fp32 (B,C,T,H,W) -> fp32 (B, F) sum-pooled trunk features."""
         m = self.res_block.inner_module
-        if STEM_DIRECT and not ops.fp32_mode() and x.shape[1] == 3 and m[0].weight.shape[0] == 64:
+        if not ops.fp32_mode() and x.shape[1] == 3 and m[0].weight.shape[0] == 64:
             # RGB padded to 16 channels (skip path) and to 4 channels (stem gather) in one pass;
             # first conv (K = 27*3 = 81): im2col tile gathered into shared memory, tensor-core GEMM, bias + ReLU
             xc, xc4 = ops.rgb_to_cl(x)
@@ -344,7 +336,7 @@ class Resnet3D(nn.Module):
         c1 = self.res_block.identity_map[1]
         pk, ps = (1, 2, 2), (2, 2, 2)                                 # AvgPool3d((1,2,2), 2): stride 2 in ALL dims
         skip = ops.conv(ops.avg_pool(xc, pk, ps), c1.weight, c1.bias)
-        if STEM_SD2 and not ops.fp32_mode() and ops.K.conv_sd2_supported(h.shape, h.shape[-1], m[2].weight.shape[0], tuple(m[2].weight.shape[2:])):
+        if not ops.fp32_mode() and ops.K.conv_sd2_supported(h.shape, h.shape[-1], m[2].weight.shape[0], tuple(m[2].weight.shape[2:])):
             # the pool keeps only the even d planes of this convolution (kernel 1, stride 2 along d): compute only those
             h = ops.conv_sd2(h, m[2].weight, m[2].bias, x_relu=True)
             h = ops.avg_pool(h, pk, (1, 2, 2), residual=skip)

@@ -127,9 +127,8 @@ int t2v_conv_fprop(const t2v_conv_geom* g, const void* x, const void* w, const f
   const bool tc_ok = igemm_fprop_supported(g);
   if ((algo == T2V_ALGO_TC || algo == T2V_ALGO_TC_GENERIC) && !tc_ok) return T2V_ERR_ARG;
   if ((epi_flags & T2V_EPI_RELU_MASK) && (algo == T2V_ALGO_SIMT || !tc_ok || !residual)) return T2V_ERR_ARG;
-  if ((epi_flags & T2V_EPI_RES_F32) && (algo == T2V_ALGO_SIMT || !tc_ok)) return T2V_ERR_ARG;
   if (algo == T2V_ALGO_SIMT || !tc_ok) return simt_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
-  if (algo != T2V_ALGO_TC_GENERIC && !(epi_flags & T2V_EPI_RES_F32) && halo_fprop_supported(g)) return halo_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
+  if (algo != T2V_ALGO_TC_GENERIC && halo_fprop_supported(g)) return halo_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
   return igemm_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
 }
 

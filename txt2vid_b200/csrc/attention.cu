@@ -597,8 +597,7 @@ int t2v_attention_fwd(const void* theta, const void* phi, const void* g, void* o
   p.phi = reinterpret_cast<const __nv_bfloat16*>(phi);
   p.g = reinterpret_cast<const __nv_bfloat16*>(g);
   p.o = reinterpret_cast<__nv_bfloat16*>(o);
-  static const bool fast_off = getenv("T2V_ATTN_GENERIC") != nullptr;
-  if (!fast_off && attn_fast_cfg(p)) {          // (two queries per thread over grid.y: any number of queries)
+  if (attn_fast_cfg(p)) {          // (two queries per thread over grid.y: any number of queries)
     const size_t sm = sizeof(float4) * (size_t)p.Kp * 5;
     if (sm <= 200 * 1024) {
       cudaFuncSetAttribute(attn_fwd_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
@@ -630,8 +629,7 @@ int t2v_attention_bwd(const void* theta, const void* phi, const void* g, const v
   p.dtheta = reinterpret_cast<__nv_bfloat16*>(dtheta);
   p.dphi = reinterpret_cast<__nv_bfloat16*>(dphi);
   p.dg = reinterpret_cast<__nv_bfloat16*>(dg);
-  static const bool fast_off = getenv("T2V_ATTN_GENERIC") != nullptr;
-  if (!fast_off && attn_fast_ok(p)) {
+  if (attn_fast_ok(p)) {
     const size_t sm = sizeof(float4) * ((size_t)p.Kp * 10 + (size_t)p.P * 5) + sizeof(float) * 3 * (size_t)p.P +
                       (size_t)p.Kp * 20 + 16;
     if (sm <= 220 * 1024) {

@@ -168,21 +168,6 @@ __global__ void multi_copy_kernel(const CopyChunk ch) {
     d[i] = s[i];
 }
 
-// Bulk host -> device copy by a few resident CTAs reading PINNED host memory over UVA and writing with streaming
-// (evict-first) stores: the input batch crosses PCIe while a training step runs, without the copy engine (whose
-// queue the step's own small transfers share) and without displacing the step's L2-resident operands.
-__global__ void __launch_bounds__(256) stream_copy_kernel(const uint4* __restrict__ src, uint4* __restrict__ dst,
-                                                         long long n16) {
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  for (; i + 3 * stride < n16; i += 4 * stride) {          // four loads in flight per thread
-    const uint4 a = __ldcs(src + i), b = __ldcs(src + i + stride), c = __ldcs(src + i + 2 * stride),
-                d = __ldcs(src + i + 3 * stride);
-    __stcs(dst + i, a); __stcs(dst + i + stride, b); __stcs(dst + i + 2 * stride, c); __stcs(dst + i + 3 * stride, d);
-  }
-  for (; i < n16; i += stride) __stcs(dst + i, __ldcs(src + i));
-}
-
 }  // namespace t2v
 
 #define ST __nv_bfloat16
@@ -271,14 +256,6 @@ int t2v_adam_step(int32_t count, float* const* host_params, const float* const* 
     count_launch();
   }
   return check_last("adam_step");
-}
-int t2v_stream_copy(const void* src, void* dst, int64_t nbytes, int32_t ctas, void* stream) {
-  if (!src || !dst || nbytes < 0 || nbytes % 16 || ctas < 1) return T2V_ERR_ARG;
-  if (nbytes == 0) return T2V_OK;
-  stream_copy_kernel<<<(unsigned)ctas, 256, 0, STREAM>>>(reinterpret_cast<const uint4*>(src),
-                                                         reinterpret_cast<uint4*>(dst), nbytes / 16);
-  count_launch();
-  return check_last("stream_copy");
 }
 int t2v_multi_copy(int32_t count, const float* const* host_src, float* const* host_dst, const int64_t* host_sizes,
                    void* stream) {

@@ -20,8 +20,7 @@
 //          An M tile is 16 LINES of 8 voxels (the 8-row groups of the canonical layout) a constant stride
 //          (the descriptor's SBO) apart: lines along h inside one plane, or along d, so no halo row is ever
 //          multiplied.  Persistent CTAs (one per SM): double-buffered halo tile, double-buffered TMEM
-//          accumulators (the epilogue of tile i overlaps the MMAs of tile i+1), and a 4-stage ring of 8 KB
-//          weight taps that is TMA-MULTICAST across a thread-block cluster (each CTA fetches 1/cs of a tap).
+//          accumulators (the epilogue of tile i overlaps the MMAs of tile i+1), and a ring of 8 KB weight taps.
 #include <cstdio>
 #include <cstdlib>
 
@@ -45,7 +44,6 @@ struct HaloWgParams {
   int xpitch_d;            // x-tile rows per d plane = (bh+2)*kXW
   int xd_mul;              // x plane of dy plane d = xd_mul * d (2: convolution with stride 2 along d)
   float* dw;
-  int debug_skip_epi;
 };
 
 __device__ __forceinline__ int halo_tap_row(int t, int kd3, int xpitch_d) {
@@ -174,7 +172,7 @@ halo_wgrad_kernel(const __grid_constant__ CUtensorMap tmDy, const __grid_constan
           uint32_t v[16];
           tmem_ld16(tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(q * p.Cout + c), v);
           tmem_ld_wait();
-          if (tap < t1 && !p.debug_skip_epi) {
+          if (tap < t1) {
             float* dst = p.dw + ((size_t)c * p.ntaps + tap) * 64 + ci;
 #pragma unroll
             for (int j = 0; j < 16; ++j) atomicAdd(dst + (size_t)j * p.ntaps * 64, __uint_as_float(v[j]));
@@ -270,7 +268,6 @@ int halo_wgrad_launch(const t2v_conv_geom* g_in, const void* dy, const void* x, 
   const t2v_conv_geom* g = &gg;
   if (!halo_wgrad_plan(g, &p, sd2)) return T2V_ERR_ARG;
   p.dw = dw;
-  { const char* e = getenv("T2V_HALO_SKIP_EPI"); p.debug_skip_epi = (e && e[0] == '1') ? 1 : 0; }
   if (!accumulate) cudaMemsetAsync(dw, 0, (size_t)g->Cout * p.ntaps * 64 * sizeof(float), stream);
   CUtensorMap tmDy, tmX;
   int rc = make_act_map(&tmDy, dy, g->N, g->D, g->H, g->W, g->Cout, 64, 8, p.bh, p.bd, 1);
@@ -311,7 +308,7 @@ struct HaloFpParams {
   int in_dmul, in_dadd;    // TMA d coordinate of a tile = in_dmul * d0 + in_dadd
   int oq_n, oq_d, oq_0;    // output plane number of (n, d)
   int wstages;
-  int t_w, t_h, t_d, tiles_total, iters, cs;
+  int t_w, t_h, t_d, tiles_total, iters;
   int th_step, td_step, tn_step;   // tile origin steps along h, d, n
   int mn, md, mh, ld, lh;          // voxel of (M tile m, line l): n0 + m*mn, d0 + m*md + l*ld, h0 + m*mh + l*lh
   int Pd, MS, LS;                  // rows per d plane, rows between M tiles, rows between lines
@@ -354,10 +351,6 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int cs = p.cs;
-  const int rank = cs > 1 ? (int)cluster_ctarank() : 0;
-  const int ncl = gridDim.x / cs, cl = blockIdx.x / cs;
-  const uint16_t mask = (uint16_t)((1u << cs) - 1u);
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -370,7 +363,7 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     }
     for (int i = 0; i < kWStages; ++i) {
       mbar_init(&w_full[i], 1);
-      mbar_init(&w_empty[i], (uint32_t)cs);
+      mbar_init(&w_empty[i], 1);
     }
     fence_barrier_init();
   }
@@ -379,7 +372,7 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     tmem_relinquish();
   }
   tc_fence_before();
-  if (cs > 1) cluster_sync_all(); else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const int acc_cols = p.np * 64;
@@ -390,27 +383,23 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       for (int it = 0; it < p.iters; ++it) {
         const int buf = it & 1;
         mbar_wait(&a_empty[buf], ((uint32_t)(it >> 1) & 1u) ^ 1u);
-        const FpTile t = fp_tile(p, (it * ncl + cl) * cs + rank);
+        const FpTile t = fp_tile(p, it * (int)gridDim.x + (int)blockIdx.x);
         mbar_expect_tx(&a_full[buf], p.a_tx);
         tma_load_5d(sA + (size_t)buf * p.a_bytes, &tmA, &a_full[buf], 0, t.w0 - 1, t.h0 - 1,
                     p.in_dmul * t.d0 + p.in_dadd, t.n0);
       }
     }
   } else if (warp == 6) {
-    // ---------------- weight ring: every CTA of the cluster fetches 1/cs of each tap and multicasts it
+    // ---------------- weight ring: one whole 64-row tap per stage
     if (lane == 0) {
       int st = 0;
       uint32_t ph = 0;
-      const int rows = 64 / cs;
       for (int it = 0; it < p.iters; ++it) {
         int t9 = 0, a_d = 0;
         for (int tap = 0; tap < p.ntaps; ++tap) {
           mbar_wait(&w_empty[st], ph ^ 1u);
           mbar_expect_tx(&w_full[st], kWTapBytes);
-          uint8_t* dst = sW + (size_t)st * kWTapBytes + (size_t)rank * rows * 128;
-          const int wtap = p.wd[a_d] * 9 + t9;
-          if (cs > 1) tma_load_2d_mc(dst, &tmW, &w_full[st], wtap * 64, rank * rows, mask);
-          else tma_load_2d(dst, &tmW, &w_full[st], wtap * 64, 0);
+          tma_load_2d(sW + (size_t)st * kWTapBytes, &tmW, &w_full[st], (p.wd[a_d] * 9 + t9) * 64, 0);
           if (++st == kWStages) { st = 0; ph ^= 1u; }
           if (++t9 == 9) { t9 = 0; ++a_d; }
         }
@@ -450,9 +439,7 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             }
           }
         }
-        if (leader) {
-          if (cs > 1) umma_commit_mc(&w_empty[st], mask); else umma_commit(&w_empty[st]);
-        }
+        if (leader) umma_commit(&w_empty[st]);
         __syncwarp();
         if (++st == kWStages) { st = 0; ph ^= 1u; }
         if (++a_w == 3) { a_w = 0; if (++a_h == 3) { a_h = 0; ++a_d; } }
@@ -470,7 +457,7 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     const int l = row >> 3, wv = row & 7;
     for (int it = 0; it < p.iters; ++it) {
       const int buf = it & 1;
-      const FpTile t = fp_tile(p, (it * ncl + cl) * cs + rank);
+      const FpTile t = fp_tile(p, it * (int)gridDim.x + (int)blockIdx.x);
       mbar_wait(&acc_full[buf], (uint32_t)(it >> 1) & 1u);
       tc_fence_after();
       for (int m = 0; m < p.np; ++m) {
@@ -534,7 +521,7 @@ halo_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     }
   }
   tc_fence_before();
-  if (cs > 1) cluster_sync_all(); else __syncthreads();
+  __syncthreads();
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc(tmem_base, p.tmem_cols);
@@ -590,7 +577,6 @@ static bool halo_fprop_plan(const t2v_conv_geom* g, HaloFpParams* p, int mode = 
     if (g->D < 2 && mode == 0) return false;
     if (g->H >= 16) {                 // 16 lines along h inside one d plane; a tile = np planes
       p->np = mode == 1 ? 1 : 2;
-      { const char* e = getenv("T2V_HALO_NP"); if (e && e[0] == '1') p->np = 1; }
       p->Pd = 18 * kXW; p->MS = (p->in_dmul ? p->in_dmul : 1) * p->Pd; p->LS = kXW;
       p->th_step = 16; p->td_step = p->np; p->tn_step = 1;
       p->md = 1; p->lh = 1;
@@ -645,26 +631,6 @@ bool halo_fprop_supported(const t2v_conv_geom* g) {
   return halo_fprop_plan(g, &p);
 }
 
-static int max_active_clusters(int cs, size_t smem) {
-  static int cache[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-  if (cache[cs] > 0) return cache[cs];
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(cs * 64), 1, 1);
-  cfg.blockDim = dim3(kFpThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  int n = 0;
-  if (cudaOccupancyMaxActiveClusters(&n, halo_fprop_kernel, &cfg) != cudaSuccess || n <= 0) {
-    cudaGetLastError();
-    n = 148 / cs / 2;     // conservative
-  }
-  cache[cs] = n;
-  return n;
-}
-
 static int halo_fprop_launch_mode(const t2v_conv_geom* g, const void* x, const void* w, const float* bias,
                                   const void* residual, void* y, uint32_t flags, cudaStream_t stream, int mode) {
   HaloFpParams p{};
@@ -678,13 +644,10 @@ static int halo_fprop_launch_mode(const t2v_conv_geom* g, const void* x, const v
   p.relu_mask = (flags & T2V_EPI_RELU_MASK) ? 1 : 0;
   const size_t smem = 2 * (size_t)p.a_bytes + p.wstages * kWTapBytes + 1024 + (8 + 2 * kWStagesMax) * 8 + 16;
   cudaFuncSetAttribute(halo_fprop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  int cs = 1;   // measured on B200: cs = 1 and 2 tie (the kernel is not weight-traffic bound), cs = 4 loses SMs
-  { const char* e = getenv("T2V_HALO_CLUSTER"); if (e && e[0] >= '1' && e[0] <= '4') cs = e[0] - '0'; if (cs == 3) cs = 2; }
-  int ncl = cs > 1 ? max_active_clusters(cs, smem) : 148;
-  const int need = (p.tiles_total + cs - 1) / cs;
-  if (ncl > need) ncl = need;
-  p.cs = cs;
-  p.iters = (p.tiles_total + ncl * cs - 1) / (ncl * cs);
+  // persistent: one CTA per SM (the weight ring is not multicast over a cluster: measured on B200, clusters of 2 tie
+  // with single CTAs because the kernel is not weight-traffic bound, and clusters of 4 lose SMs)
+  const int grid = p.tiles_total < 148 ? p.tiles_total : 148;
+  p.iters = (p.tiles_total + grid - 1) / grid;
 
   CUtensorMap tmA, tmW;
   int rc;
@@ -693,25 +656,15 @@ static int halo_fprop_launch_mode(const t2v_conv_geom* g, const void* x, const v
   else
     rc = make_act_map(&tmA, x, g->N, g->D, g->H, g->W, 64, 64, kXW, p.box_h, p.box_d, p.box_n);
   if (rc) return rc;
-  rc = make_w_map(&tmW, w, 64, g->kd * 9 * 64, 64, 64 / cs);
+  rc = make_w_map(&tmW, w, 64, g->kd * 9 * 64, 64, 64);
   if (rc) return rc;
 
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(ncl * cs), 1, 1);
-  cfg.blockDim = dim3(kFpThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
   ProfRec rec;
   if (g_prof_on)     // useful MACs: output voxels x live taps
-    prof_begin(stream, &rec, 2, 2.0 * p.N * p.D * g->H * g->W * 64.0 * 64.0 * p.ntaps, g, ncl * cs);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, halo_fprop_kernel, tmA, tmW, p);
+    prof_begin(stream, &rec, 2, 2.0 * p.N * p.D * g->H * g->W * 64.0 * 64.0 * p.ntaps, g, grid);
+  halo_fprop_kernel<<<grid, kFpThreads, smem, stream>>>(tmA, tmW, p);
   if (g_prof_on) prof_end(stream, &rec);
   count_launch();
-  if (e != cudaSuccess) { cudaGetLastError(); return T2V_ERR_LAUNCH; }
   return check_last("halo_fprop");
 }
 

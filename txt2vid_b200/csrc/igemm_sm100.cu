@@ -42,7 +42,7 @@ struct IgemmParams {
   const float* bias;
   const __nv_bfloat16* residual;
   void* out;
-  int out_f32, relu, relu_mask, res_f32;
+  int out_f32, relu, relu_mask;
   // fused ConvLSTM cell epilogue (columns gate-interleaved per 32 hidden units: tile = [i | f | g | o] x 32)
   int lstm, lstm_t, lstm_steps, lstm_plane;
   const float* c_prev;
@@ -52,7 +52,7 @@ struct IgemmParams {
   __nv_bfloat16* h_merged;
   // wgrad only
   float* dw;
-  int taps_total, splits, tiles_total, atomic_out, tap_fast, col_fast;
+  int taps_total, splits, tiles_total, atomic_out;
 };
 
 static constexpr int kThreads = 192;
@@ -76,21 +76,7 @@ T2V_DEVINL void fprop_epilogue16(const IgemmParams& p, const uint32_t (&v)[16], 
       f[j] += b.x; f[j + 1] += b.y; f[j + 2] += b.z; f[j + 3] += b.w;
     }
   }
-  if (p.residual != nullptr && p.res_f32) {
-    // fp32 residual / ReLU reference (fp32 activation storage on the tensor-pipe engine)
-    const float4* rp = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.residual) +
-                                                       pos * p.Cout + col);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float4 r4 = rp[j];
-      if (p.relu_mask) {
-        f[4 * j + 0] = r4.x > 0.f ? f[4 * j + 0] : 0.f; f[4 * j + 1] = r4.y > 0.f ? f[4 * j + 1] : 0.f;
-        f[4 * j + 2] = r4.z > 0.f ? f[4 * j + 2] : 0.f; f[4 * j + 3] = r4.w > 0.f ? f[4 * j + 3] : 0.f;
-      } else {
-        f[4 * j + 0] += r4.x; f[4 * j + 1] += r4.y; f[4 * j + 2] += r4.z; f[4 * j + 3] += r4.w;
-      }
-    }
-  } else if (p.residual != nullptr) {
+  if (p.residual != nullptr) {
     const uint4* rp = reinterpret_cast<const uint4*>(p.residual + pos * p.Cout + col);
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
@@ -186,9 +172,9 @@ T2V_DEVINL void lstm_epilogue_row(const IgemmParams& p, uint32_t taddr, size_t p
 }
 
 // PERSISTENT: gridDim.x CTAs (a multiple of the SM count, or every tile when there are few) walk the output tiles
-// tile = blockIdx.x, + gridDim.x, ...  Column tile fastest (col_fast): the CTAs running at the same time share the
-// ACTIVATION tile, which is then read from DRAM once instead of once per column tile (the weights of a layer, <= 19 MB,
-// stay in the 126 MB L2 either way); m fastest was round 1's order.
+// tile = blockIdx.x, + gridDim.x, ...  Column tile fastest: the CTAs running at the same time share the ACTIVATION
+// tile, which is then read from DRAM once instead of once per column tile (the weights of a layer, <= 19 MB, stay in
+// the 126 MB L2 either way).
 // The TMA ring runs ahead ACROSS tiles (no pipeline fill / drain per tile), the accumulator is double buffered in
 // TMEM (2 x BN columns): the MMA warp starts tile i+1 while the epilogue warps drain tile i, and barrier init /
 // TMEM allocation / descriptor prefetch are paid once per CTA instead of once per 128-row tile.
@@ -208,9 +194,8 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int mtiles = p.tn * p.td * p.th * p.tw;
-  const int total = p.tiles_total;                  // mtiles * column tiles
-  const int ncols = total / mtiles;
+  const int total = p.tiles_total;                  // m tiles * column tiles
+  const int ncols = total / (p.tn * p.td * p.th * p.tw);
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -245,8 +230,8 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       uint32_t phase = 0;
       const int nkw = p.hi_w - p.lo_w, nkh = p.hi_h - p.lo_h;
       for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        int mt = p.col_fast ? tile / ncols : tile % mtiles;
-        const int col0 = (p.col_fast ? tile % ncols : tile / mtiles) * p.BN;
+        int mt = tile / ncols;
+        const int col0 = (tile % ncols) * p.BN;
         const int tw_i = mt % p.tw; mt /= p.tw;
         const int th_i = mt % p.th; mt /= p.th;
         const int td_i = mt % p.td; mt /= p.td;
@@ -324,8 +309,8 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     const int id = r % p.bd; r /= p.bd;
     int it = 0;
     for (int tile = blockIdx.x; tile < total; tile += gridDim.x, ++it) {
-      int mt = p.col_fast ? tile / ncols : tile % mtiles;
-      const int col0 = (p.col_fast ? tile % ncols : tile / mtiles) * p.BN;
+      int mt = tile / ncols;
+      const int col0 = (tile % ncols) * p.BN;
       const int tw_i = mt % p.tw; mt /= p.tw;
       const int th_i = mt % p.th; mt /= p.th;
       const int td_i = mt % p.td; mt /= p.td;
@@ -390,9 +375,9 @@ igemm_fprop_simple_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_
   const int lane = threadIdx.x & 31;
 
   // tile coordinates (1-D grid; same order as the persistent kernel)
-  const int mtiles_ = p.tn * p.td * p.th * p.tw, ncols_ = p.tiles_total / mtiles_;
-  int mt = p.col_fast ? (int)blockIdx.x / ncols_ : (int)blockIdx.x % mtiles_;
-  const int col0 = (p.col_fast ? (int)blockIdx.x % ncols_ : (int)blockIdx.x / mtiles_) * p.BN;
+  const int ncols = p.tiles_total / (p.tn * p.td * p.th * p.tw);
+  int mt = (int)blockIdx.x / ncols;
+  const int col0 = ((int)blockIdx.x % ncols) * p.BN;
   const int tw_i = mt % p.tw; mt /= p.tw;
   const int th_i = mt % p.th; mt /= p.th;
   const int td_i = mt % p.td; mt /= p.td;
@@ -510,21 +495,7 @@ igemm_fprop_simple_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_
             f[j] += b.x; f[j + 1] += b.y; f[j + 2] += b.z; f[j + 3] += b.w;
           }
         }
-        if (p.residual != nullptr && p.res_f32) {
-          // fp32 residual / ReLU reference (fp32 activation storage: the 1e-3 parity mode)
-          const float4* rp = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.residual) +
-                                                             pos * p.Cout + col);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 r4 = rp[j];
-            if (p.relu_mask) {
-              f[4 * j + 0] = r4.x > 0.f ? f[4 * j + 0] : 0.f; f[4 * j + 1] = r4.y > 0.f ? f[4 * j + 1] : 0.f;
-              f[4 * j + 2] = r4.z > 0.f ? f[4 * j + 2] : 0.f; f[4 * j + 3] = r4.w > 0.f ? f[4 * j + 3] : 0.f;
-            } else {
-              f[4 * j + 0] += r4.x; f[4 * j + 1] += r4.y; f[4 * j + 2] += r4.z; f[4 * j + 3] += r4.w;
-            }
-          }
-        } else if (p.residual != nullptr) {
+        if (p.residual != nullptr) {
           const uint4* rp = reinterpret_cast<const uint4*>(p.residual + pos * p.Cout + col);
 #pragma unroll
           for (int j = 0; j < 2; ++j) {
@@ -592,8 +563,8 @@ igemm_wgrad_kernel(const __grid_constant__ CUtensorMap tmDy, const __grid_consta
   // dram__bytes_read = 2-3x the operand bytes.
   const int nkw = p.hi_w - p.lo_w, nkh = p.hi_h - p.lo_h;
   const int ntaps_live = nkw * nkh * (p.hi_d - p.lo_d);
-  const int split = p.tap_fast ? (int)blockIdx.z / ntaps_live : (int)blockIdx.z % p.splits;
-  int t = p.tap_fast ? (int)blockIdx.z % ntaps_live : (int)blockIdx.z / p.splits;
+  const int split = (int)blockIdx.z / ntaps_live;
+  int t = (int)blockIdx.z % ntaps_live;
   const int a_w = t % nkw + p.lo_w; t /= nkw;
   const int a_h = t % nkh + p.lo_h; t /= nkh;
   const int a_d = t + p.lo_d;
@@ -748,6 +719,13 @@ void prof_read(double* out, int nkinds) {
   g_prof.clear();
 }
 
+// fprop: shared memory of a CTA on small-stage (<= 12 KB) problems of more than four waves, one tile / persistent
+static constexpr uint32_t kFpropSmallSmemKB = 32, kFpropSmallSmemKBPersist = 48;
+// fprop: the persistent kernel runs when a tile's K (main + fused skip) reaches this many channels
+static constexpr int kFpropPersistMinK = 512;
+// wgrad: go beyond two waves of 148 only while each CTA still sums this many position boxes
+static constexpr int kWgradMinBoxes = 32;
+
 static int env_int(const char* name, int dflt) {
   const char* e = getenv(name);
   return e ? atoi(e) : dflt;
@@ -833,9 +811,8 @@ int igemm_fprop_launch_aux(const t2v_conv_geom* g, const void* x, const void* w,
   p.th = (g->H + p.bh - 1) / p.bh; p.tw = (g->W + p.bw - 1) / p.bw;
   p.BN = g->Cout >= 128 ? 128 : g->Cout;
   const int mtiles_total = p.tn * p.td * p.th * p.tw;
-  static const int adapt_bn = env_int("T2V_FPROP_ADAPT_BN", 1), two_cta = env_int("T2V_FPROP_2CTA", 1);
   // small problems: narrower N tiles -> more CTAs (the kernel is load-latency bound there, not tensor bound)
-  if (adapt_bn && !lstm)
+  if (!lstm)
     while (p.BN > 64 && p.BN % 32 == 0 && mtiles_total * ((g->Cout + p.BN - 1) / p.BN) < 120) p.BN /= 2;
   p.cblocks = g->Cin / BLOCK_K;
   p.num_k_blocks = ntaps * p.cblocks;
@@ -849,18 +826,15 @@ int igemm_fprop_launch_aux(const t2v_conv_geom* g, const void* x, const void* w,
   // many CTAs: cap shared memory at half an SM so that two CTAs are co-resident and one CTA's prologue /
   // epilogue overlaps the other's main loop (TMEM: 2 x BN <= 512 columns)
   const int total_ctas = mtiles_total * ((g->Cout + p.BN - 1) / p.BN);
-  uint32_t budget = (two_cta && total_ctas > 222) ? 106496u : 196608u;
+  uint32_t budget = total_ctas > 222 ? 106496u : 196608u;
   // short K loops over small tiles are latency bound per CTA: trade pipeline depth for residency (measured:
   // 32->32 channels at 64x64, 9 k-blocks of 10 KB: 0.166 -> 0.082 ms with 3 stages and 6 CTAs per SM)
-  static const int small_kb = env_int("T2V_FPROP_SMALL_SMEM_KB", 32);
-  // persistent + double-buffered accumulator: more than one wave of tiles and K >= T2V_FPROP_PERSIST_MIN_K per tile
+  // persistent + double-buffered accumulator: more than one wave of tiles and K >= kFpropPersistMinK per tile
   // (measured in situ at b = 2048: 64..1024-channel 3x3(x3) layers +15..30 %, 1x1 / 16-32-channel layers -10 %)
-  static const int persist_env = env_int("T2V_FPROP_PERSIST", 1), persist_min_k = env_int("T2V_FPROP_PERSIST_MIN_K", 512);
-  const int persist = lstm != nullptr ||        // (the fused LSTM epilogue lives in the persistent kernel)
-      (persist_env && total_ctas > 296 && (p.num_k_blocks + p.aux_k_blocks) * BLOCK_K >= persist_min_k);
-  static const int small_kb_p = env_int("T2V_FPROP_SMALL_SMEM_KB_PERSIST", 48);
-  if (small_kb > 0 && p.stage_bytes <= 12288u && total_ctas > 4 * 148)
-    budget = (uint32_t)(persist ? small_kb_p : small_kb) * 1024u;
+  const bool persist = lstm != nullptr ||        // (the fused LSTM epilogue lives in the persistent kernel)
+      (total_ctas > 296 && (p.num_k_blocks + p.aux_k_blocks) * BLOCK_K >= kFpropPersistMinK);
+  if (p.stage_bytes <= 12288u && total_ctas > 4 * 148)
+    budget = (persist ? kFpropSmallSmemKBPersist : kFpropSmallSmemKB) * 1024u;
   int stages = (int)(budget / p.stage_bytes);
   if (stages < 2) stages = 2;
   if (stages > 8) stages = 8;
@@ -878,10 +852,7 @@ int igemm_fprop_launch_aux(const t2v_conv_geom* g, const void* x, const void* w,
   p.out_f32 = (flags & T2V_EPI_OUT_F32) ? 1 : 0;
   p.relu = (flags & T2V_EPI_RELU) ? 1 : 0;
   p.relu_mask = (flags & T2V_EPI_RELU_MASK) ? 1 : 0;
-  p.res_f32 = (flags & T2V_EPI_RES_F32) ? 1 : 0;
   p.tiles_total = total_ctas;
-  static const int col_fast = env_int("T2V_FPROP_COL_FAST", 1);
-  p.col_fast = col_fast;
   if (lstm) {
     p.lstm = 1; p.lstm_t = lstm->t; p.lstm_steps = lstm->steps; p.lstm_plane = g->D * g->H * g->W;
     p.c_prev = lstm->c_prev; p.c_out = lstm->c_out; p.gates_out = lstm->gates;
@@ -923,26 +894,24 @@ int igemm_fprop_launch_aux(const t2v_conv_geom* g, const void* x, const void* w,
     return check_last("igemm_fprop");
   }
   // persistent grid: as many CTAs as stay resident (shared memory, TMEM columns, threads), each walking
-  // tiles blockIdx.x, + gridDim.x, ...; T2V_FPROP_PERSIST=0 launches one CTA per tile (the round-1 schedule)
+  // tiles blockIdx.x, + gridDim.x, ...
   int grid_x = total_ctas;
   auto launch = [&](auto kern) {
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (persist) {
-      static int regs_cached[3] = {0, 0, 0};
-      int& rc_ = regs_cached[BLOCK_K == 64 ? 0 : (BLOCK_K == 32 ? 1 : 2)];
-      if (rc_ == 0) {
-        cudaFuncAttributes fa{};
-        cudaFuncGetAttributes(&fa, kern);
-        rc_ = fa.numRegs > 0 ? fa.numRegs : 96;
-      }
-      const int regs = (rc_ + 7) & ~7;                                                  // allocation granularity
-      int per_sm = 65536 / (regs * kThreads);                                           // registers ...
-      if (per_sm > (int)((228u * 1024u) / (smem + 1024u))) per_sm = (int)((228u * 1024u) / (smem + 1024u));
-      if (per_sm > 2048 / kThreads) per_sm = 2048 / kThreads;                           // ... shared memory, threads
-      if (per_sm > (int)(512u / p.tmem_cols)) per_sm = (int)(512u / p.tmem_cols);      // ... and TMEM columns
-      if (per_sm < 1) per_sm = 1;
-      if (grid_x > 148 * per_sm) grid_x = 148 * per_sm;
+    static int regs_cached[3] = {0, 0, 0};
+    int& rc_ = regs_cached[BLOCK_K == 64 ? 0 : (BLOCK_K == 32 ? 1 : 2)];
+    if (rc_ == 0) {
+      cudaFuncAttributes fa{};
+      cudaFuncGetAttributes(&fa, kern);
+      rc_ = fa.numRegs > 0 ? fa.numRegs : 96;
     }
+    const int regs = (rc_ + 7) & ~7;                                                    // allocation granularity
+    int per_sm = 65536 / (regs * kThreads);                                             // registers ...
+    if (per_sm > (int)((228u * 1024u) / (smem + 1024u))) per_sm = (int)((228u * 1024u) / (smem + 1024u));
+    if (per_sm > 2048 / kThreads) per_sm = 2048 / kThreads;                             // ... shared memory, threads
+    if (per_sm > (int)(512u / p.tmem_cols)) per_sm = (int)(512u / p.tmem_cols);        // ... and TMEM columns
+    if (per_sm < 1) per_sm = 1;
+    if (grid_x > 148 * per_sm) grid_x = 148 * per_sm;
     static const int dbg = env_int("T2V_DEBUG_LAUNCH", 0);
     if (dbg)
       fprintf(stderr, "igemm_fprop N%d D%d H%d W%d Cin%d Cout%d k%d%d%d: tiles %d grid %d stages %d stage_bytes %u smem %zu "
@@ -980,13 +949,11 @@ int igemm_wgrad_launch(const t2v_conv_geom* g, const void* dy, const void* x, fl
   const int base_ctas = mtiles * ntiles * ntaps;
   // two CTAs per SM (shared memory capped at half an SM: one CTA's prologue / atomics epilogue overlaps the
   // other's main loop): fill at most two FULL waves of 2 x 148 so that no nearly empty extra wave runs
-  static const int two_cta = env_int("T2V_WGRAD_2CTA", 1);
-  const int slots = two_cta ? 2 * 148 : 148;
-  int splits = (2 * slots) / base_ctas;
+  int splits = (2 * 2 * 148) / base_ctas;
   // every split adds a full Cout x taps x Cin round of fp32 atomics: only go beyond two waves of 148 when each
-  // CTA still sums >= 32 position boxes (position-heavy layers), else the atomics of weight-heavy layers dominate
-  static const int min_boxes = env_int("T2V_WGRAD_MIN_BOXES", 32);
-  if (splits < 1 || p.tiles_total / (splits < 1 ? 1 : splits) < min_boxes) splits = (2 * 148) / base_ctas;
+  // CTA still sums >= kWgradMinBoxes position boxes (position-heavy layers), else the atomics of weight-heavy layers
+  // dominate
+  if (splits < 1 || p.tiles_total / splits < kWgradMinBoxes) splits = (2 * 148) / base_ctas;
   const int max_splits = (p.tiles_total + 3) / 4;  // keep >= 4 k-blocks per CTA
   if (splits > max_splits) splits = max_splits;
   if (splits < 1) splits = 1;
@@ -994,14 +961,12 @@ int igemm_wgrad_launch(const t2v_conv_geom* g, const void* dy, const void* x, fl
   p.a_bytes = 2u * kWgradPos * 128u;
   p.b_bytes = (uint32_t)(p.BN / 64) * kWgradPos * 128u;
   p.stage_bytes = p.a_bytes + p.b_bytes;
-  int stages = (int)((two_cta ? 106496u : 196608u) / p.stage_bytes);
+  int stages = (int)(106496u / p.stage_bytes);
   if (stages > 8) stages = 8;
   p.stages = stages;
   p.idesc = make_idesc_bf16(128, (uint32_t)p.BN, 1, 1);
   p.tmem_cols = (uint32_t)(p.BN < 32 ? 32 : p.BN);
   p.dw = dw;
-  static const int tap_fast = env_int("T2V_WGRAD_TAP_FAST", 1);
-  p.tap_fast = tap_fast;
   p.atomic_out = (splits > 1 || accumulate) ? 1 : 0;
 
   const size_t dw_elems = (size_t)g->Cout * p.taps_total * g->Cin;

@@ -337,8 +337,7 @@ template <typename ST>
 static int lstm_fwd_impl(LstmSeq p, cudaStream_t s) {
   if (p.H % 32 || p.H > 1024 || p.B <= 0 || p.L <= 0 || p.ndir < 1 || p.ndir > 2) return T2V_ERR_ARG;
   dim3 grid((p.B + kLstmBT - 1) / kLstmBT, p.ndir, 1);
-  static const int use_smem = [] { const char* e = getenv("T2V_LSTM_SMEM"); return e ? atoi(e) : 1; }();
-  if (use_smem && sizeof(ST) == 2 && p.H == 128) {            // bf16 storage mode: recurrent weights resident in smem
+  if (sizeof(ST) == 2 && p.H == 128) {            // bf16 storage mode: recurrent weights resident in smem
     const size_t smem = (size_t)p.H * p.H * 8 + sizeof(float) * kLstmBT * p.H;
     cudaFuncSetAttribute(lstm_seq_fwd_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     lstm_seq_fwd_smem_kernel<<<grid, kLstmSmemThreads, smem, s>>>(p);

@@ -4,7 +4,7 @@
 // fp32 operands (T2V_EPI_IN_F32 / T2V_ALGO_SIMT_F32) -- as the convolution of the fp32 PARITY mode: exact fp32
 // products, fp32 accumulation flushed once per tap (chains of <= Cin FMAs), i.e. the reference's own numerics.  The
 // tensor pipe cannot give that: its fp32 accumulator truncates on every MMA, which costs ~3e-5 relative on the
-// K = 9216 layers however finely the operands are split (measured, scripts/debug_fp32_conv.py).
+// K = 9216 layers however finely the operands are split (measured: profiles/r02_fp32_engine_accuracy.txt).
 #include "t2v_common.cuh"
 
 namespace t2v {

@@ -8,8 +8,7 @@
 //   * relativistic / Wasserstein loss reduction over all pyramid levels and prediction pairs in ONE launch forward and
 //     ONE backward (gan/losses.py:55-85, gan/cond_gan.py:51-61);
 //   * gradient-penalty arithmetic: per-sample interpolation (gan/losses.py:140-145) and the fp32 dot / scale kernels
-//     behind sum ||g||^2 and its derivative (losses.py:180-186);
-//   * bf16x3 operand split of fp32 activations for the fp32 parity mode of the tcgen05 engine.
+//     behind sum ||g||^2 and its derivative (losses.py:180-186).
 #include "t2v_common.cuh"
 
 namespace t2v {
@@ -17,46 +16,6 @@ namespace t2v {
 static inline unsigned nblocks(long long n, int per) {
   long long b = (n + per - 1) / per;
   return (unsigned)(b < 1 ? 1 : b);
-}
-
-// ------------------------------------------------------------------------------------ bf16 operand split
-// x fp32 [rows][C] -> bf16 parts a = bf16(x), b = bf16(x - a), c = bf16(x - a - b) (x = a + b + c to 24 bits).
-// terms = 3 (16 bits per operand): products a a' + b a' + a b'
-//   layout 0: out [rows][3C]  = [a | b | a]         (K-concatenated A operand of fprop / dgrad; weights [a | a | b])
-//   layout 1: out [3*rows][C] = [a ; b ; a]         (position-concatenated dy operand of wgrad)
-//   layout 2: out [3*rows][C] = [a ; a ; b]         (position-concatenated x operand of wgrad)
-// terms = 6 (24 bits per operand = fp32 operands): a a' + b a' + a b' + c a' + a c' + b b'
-//   layout 0 / 1: [a | b | a | c | a | b],  layout 2 (and the weight packs): [a | a | b | a | c | b]
-// so that sum_k a_k b_k over the concatenated axis is the fp32 product on the bf16 tensor pipe with fp32
-// accumulation (dropped terms b c', c b', c c' <= 2^-24 relative).
-__global__ void split_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, long long rows, int C,
-                             int layout, int terms, long long total4) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const long long r = i / c4;
-  const int c = (int)(i % c4) * 4;
-  const float4 v = *reinterpret_cast<const float4*>(x + r * C + c);
-  const float f[4] = {v.x, v.y, v.z, v.w};
-  float pa[4], pb[4], pc[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    pa[j] = bf2f(f2bf(f[j]));
-    const float r1 = f[j] - pa[j];                 // exact
-    pb[j] = bf2f(f2bf(r1));
-    pc[j] = r1 - pb[j];                            // exact; fits bf16 up to the last fp32 bits
-  }
-  uint2 P[3];
-  P[0] = make_uint2(pack_bf16x2(pa[0], pa[1]), pack_bf16x2(pa[2], pa[3]));
-  P[1] = make_uint2(pack_bf16x2(pb[0], pb[1]), pack_bf16x2(pb[2], pb[3]));
-  P[2] = make_uint2(pack_bf16x2(pc[0], pc[1]), pack_bf16x2(pc[2], pc[3]));
-  // part index per segment: x-side order (layouts 0, 1) and w-side order (layout 2)
-  const int xs[6] = {0, 1, 0, 2, 0, 1}, ws[6] = {0, 0, 1, 0, 2, 1};
-  const long long seg = layout == 0 ? (long long)C : rows * C;
-  __nv_bfloat16* o = layout == 0 ? out + r * terms * C + c : out + r * C + c;
-#pragma unroll
-  for (int t = 0; t < 6; ++t)
-    if (t < terms) *reinterpret_cast<uint2*>(o + t * seg) = P[layout == 2 ? ws[t] : xs[t]];
 }
 
 // ------------------------------------------------------------------------------------ 1x2x2 max-pool with arg-max
@@ -345,19 +304,6 @@ using namespace t2v;
 #define STREAM reinterpret_cast<cudaStream_t>(stream)
 
 extern "C" {
-
-int t2v_split_bf16(const float* x, void* out, int64_t rows, int32_t C, int32_t layout, int32_t terms, void* stream) {
-  if (!x || !out || C % 4 || layout < 0 || layout > 2 || (terms != 3 && terms != 6)) return T2V_ERR_ARG;
-  const long long total4 = rows * C / 4;
-  if (total4 == 0) return T2V_OK;
-  split_kernel<<<nblocks(total4, 256), 256, 0, STREAM>>>(x, reinterpret_cast<__nv_bfloat16*>(out), rows, C, layout,
-                                                         terms, total4);
-  count_launch();
-  return check_last("split_bf16");
-}
-int t2v_split_bf16x3(const float* x, void* out, int64_t rows, int32_t C, int32_t layout, void* stream) {
-  return t2v_split_bf16(x, out, rows, C, layout, 3, stream);
-}
 
 int t2v_maxpool122_fwd(const float* x, float* y, void* idx, int64_t maps, int32_t H, int32_t W, int32_t c,
                        void* stream) {

@@ -269,32 +269,4 @@ T2V_DEVINL void umma_bf16_ss2(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uin
       : "memory");
 }
 
-// ---------------------------------------------------------------- thread-block clusters
-T2V_DEVINL uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-T2V_DEVINL void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA load multicast to the CTAs in `mask` (same smem offset and same mbarrier offset in each of them)
-T2V_DEVINL void tma_load_2d_mc(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// tcgen05.commit whose mbarrier arrive is multicast to the same barrier offset in every CTA of `mask`
-T2V_DEVINL void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(mask)
-      : "memory");
-}
-
 }  // namespace t2v

@@ -3,8 +3,6 @@ txt2vid/data/__init__.py:260-355 Vocab / collate_fn), a pinned-memory prefetcher
 `data_prefetcher.next()` contract (:131-156), and synthetic batches of the shapes SURVEY.md 8(d) names.
 The reference's file/LMDB datasets, DALI hooks and caches are out of scope (SURVEY.md 2.1 rows 15-17).
 """
-import os
-
 import torch
 
 
@@ -91,10 +89,9 @@ class data_prefetcher(object):
     them with the graph replay that follows (100-115 ms); a host-side wait on the PREVIOUS step's event stalls the
     host, which must stay more than one step ahead of the device for back-to-back graph launches (100 ms); with the
     guard two steps back the event has always fired and the copies overlap (91 ms)."""
-    CHUNK_BYTES = int(os.environ.get("T2V_PF_CHUNK_MB", "48")) << 20
-    SLOTS = int(os.environ.get("T2V_PF_SLOTS", "4"))
+    CHUNK_BYTES = 48 << 20
+    SLOTS = 4
     GUARD = "host"
-    SM_COPY_CTAS = int(os.environ.get("T2V_PF_SM_COPY_CTAS", "0"))   # > 0: bulk copy by an SM kernel over UVA (experimental)
 
     def __init__(self, loader, device=None, normalize=True):
         # normalize=False: uint8 frames are handed out as stored; the consumer normalises them where it needs them
@@ -127,10 +124,6 @@ class data_prefetcher(object):
         # replayed graph for its whole duration (step 100.6 -> 117.5 ms); the same bytes in <= 64 MB pieces overlap
         # (102.4 ms): scripts/h2d_probe.py
         nbytes = t.numel() * t.element_size()
-        if self.SM_COPY_CTAS > 0 and nbytes >= (1 << 20) and nbytes % 16 == 0 and t.is_contiguous():
-            from . import kernels as K
-            K.stream_copy(t, buf, self.SM_COPY_CTAS)
-            return buf
         pieces = min(t.size(0), -(-nbytes // self.CHUNK_BYTES)) if t.dim() > 0 and t.is_contiguous() else 1
         if pieces <= 1:
             buf.copy_(t, non_blocking=True)

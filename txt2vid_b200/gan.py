@@ -188,10 +188,6 @@ def gradient_penalty(discrim, real_x=None, real_xbar=None, fake_x=None, fake_xba
     return out
 
 
-import os as _os
-PAIR_D_STEP = _os.environ.get("T2V_PAIR_D_STEP", "1") == "1"   # batch the real / fake trunk passes of the D step
-
-
 def _zero_grad(module):
     """module.zero_grad() of cond_gan.py:91,157; the product modules' conv weights keep persistent gradient buffers
     that the weight-gradient kernels accumulate into (ops.zero_grads)."""
@@ -236,7 +232,7 @@ class CondGan(object):
         fake_pred = real_pred = l = None
         if real_cond is not None and fake_cond is not None:
             pair = loss is not None and hasattr(discrim, "forward_pair") and real_mapping is None \
-                and fake_mapping is None and PAIR_D_STEP
+                and fake_mapping is None
             if pair:       # (x_r, c_r) and (x_f, c_r) through the shared trunk in one pass (no normalisation in D)
                 real_cc, fake_cc = discrim.forward_pair(x_a=real, x_b=fake, cond_a=real_cond, cond_b=real_cond)
             else:
@@ -262,7 +258,7 @@ class CondGan(object):
                     l = (l_u + l_c) / 2.0
         else:
             if real is not None and fake is not None and loss is not None and hasattr(discrim, "forward_pair") \
-                    and real_mapping is None and fake_mapping is None and PAIR_D_STEP:
+                    and real_mapping is None and fake_mapping is None:
                 ra, fa = discrim.forward_pair(x_a=real, x_b=fake)
                 real_pred, fake_pred = [r[0] for r in ra], [f[0] for f in fa]
             else:

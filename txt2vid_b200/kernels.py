@@ -6,7 +6,6 @@ only talks to the GPU through these functions.  There is no CPU path: every func
 non-CUDA tensors (tests/cpu_kernels.py is a test-only stand-in used to check the autograd formulas).
 """
 import ctypes
-import os
 
 import torch
 
@@ -18,8 +17,8 @@ F32 = torch.float32
 
 # Activation storage type of the tensors the wrappers CREATE at fp32 boundaries (layout conversion, operand packs,
 # broadcast / render / LSTM outputs).  bf16 is the product; fp32 is the parity mode of BASELINE's north_star (1e-3 on
-# losses and gradients): same kernels instantiated for float storage, and the tcgen05 engine fed with bf16 hi / lo
-# operand splits (see conv_fprop).  Elementwise wrappers follow the dtype of their input.
+# losses and gradients): same kernels instantiated for float storage, and the convolutions on exact fp32 FMAs on the
+# CUDA cores (see conv_fprop).  Elementwise wrappers follow the dtype of their input.
 STORE = BF16
 
 
@@ -49,33 +48,11 @@ def _act(*ts):
         assert t is None or (t.dtype in (BF16, F32) and t.is_contiguous()), (None if t is None else (t.dtype, t.shape))
 
 
-# fp32 storage mode, convolution engine:
-#   "ffma" (default): fp32 operands, exact fp32 FMAs on the CUDA cores (simt_conv.cu, T2V_EPI_IN_F32): the reference's
-#           own numerics, ~1e-6 per layer -- what the 1e-3 bar on GRADIENTS needs on this network (a forward
-#           deviation of 5e-5 already moves the generator's gradients by 5e-3 through ReLU / BatchNorm, measured);
-#   "tc":   the tcgen05 engine on bf16 part splits of the fp32 operands (SPLIT_TERMS products per fp32 product;
-#           3: 16 bits per operand, 6: 24 bits).  Operands are then exact, but the tensor pipe's fp32 accumulator
-#           truncates on every MMA: 7e-6 relative at K = 1024, 3e-5 at K = 9216, WORSE with more terms (longer
-#           chains) -- scripts/debug_fp32_conv.py, profiles/r02_fp32_engine_accuracy.txt.
-FP32_ENGINE = os.environ.get("T2V_FP32_ENGINE", "ffma")
-SPLIT_TERMS = int(os.environ.get("T2V_FP32_SPLIT", "3"))
-assert SPLIT_TERMS in (3, 6) and FP32_ENGINE in ("ffma", "tc")
-
-
-def split3(x, layout):
-    """fp32 (..., C) -> bf16 part split for the tensor pipe (SPLIT_TERMS = T segments): layout 0 (..., T*C) along the
-    channels; 1 / 2: (T*N, ..., C) along the leading dim, activation-side / weight-side part order."""
-    require_cuda(x)
-    assert x.dtype == F32 and x.is_contiguous()
-    C = x.shape[-1]
-    rows = x.numel() // C
-    T = SPLIT_TERMS
-    if layout == 0:
-        out = torch.empty(tuple(x.shape[:-1]) + (T * C,), device=x.device, dtype=BF16)
-    else:
-        out = torch.empty((T * x.shape[0],) + tuple(x.shape[1:]), device=x.device, dtype=BF16)
-    check(lib().t2v_split_bf16(ptr(x), ptr(out), rows, C, layout, T, stream()), "t2v_split_bf16")
-    return out
+# fp32 storage mode, convolution engine: fp32 operands, exact fp32 FMAs on the CUDA cores (simt_conv.cu,
+# T2V_EPI_IN_F32): the reference's own numerics, ~1e-6 per layer -- what the 1e-3 bar on GRADIENTS needs on this
+# network (a forward deviation of 5e-5 already moves the generator's gradients by 5e-3 through ReLU / BatchNorm,
+# measured).  The tensor pipe on bf16 part splits of the fp32 operands does not reach it: its fp32 accumulator
+# truncates on every MMA (7e-6 relative at K = 1024, 3e-5 at K = 9216; profiles/r02_fp32_engine_accuracy.txt).
 
 
 def _geom(N, D, H, W, Cin, Cout, k):
@@ -90,30 +67,20 @@ def _i32(*vals):
 # ------------------------------------------------------------------------------------- conv engine
 def conv_fprop(x, w, bias=None, residual=None, k=(3, 3, 3), relu=False, out_f32=False, algo=0):
     """x (N,D,H,W,Cin) bf16, w (Cout,taps,Cin) bf16 -> y (N,D,H,W,Cout) bf16|f32.
-    fp32 storage: x fp32, w the K-concatenated pack (Cout,taps,T*Cin) of pack_weight, T = SPLIT_TERMS -> y fp32 (residual fp32)."""
+    fp32 storage: x, w (and residual) fp32 -> y fp32."""
     require_cuda(x, w, bias, residual)
     N, D, H, W, Cin = x.shape
     Cout = w.shape[0]
-    f32 = x.dtype == F32
-    ffma = f32 and w.dtype == F32                 # fp32 parity mode on exact fp32 FMAs
-    if ffma:
-        out_f32 = True
-        assert residual is None or residual.dtype == F32
-    elif f32:
-        assert w.shape[2] == SPLIT_TERMS * Cin, (w.shape, Cin)
-        x = split3(x, 0)
-        Cin, out_f32 = SPLIT_TERMS * Cin, True
-        assert residual is None or residual.dtype == F32
+    f32 = x.dtype == F32                          # fp32 parity mode on exact fp32 FMAs
+    if f32:
+        out_f32, algo = True, _lib.ALGO_SIMT
     assert w.shape[1] == k[0] * k[1] * k[2] and w.shape[2] == Cin, (w.shape, k, Cin)
-    assert x.is_contiguous() and w.is_contiguous() and (ffma or (x.dtype == BF16 and w.dtype == BF16))
+    assert x.is_contiguous() and w.is_contiguous() and w.dtype == x.dtype
     assert bias is None or (bias.dtype == F32 and bias.numel() == Cout)
     assert residual is None or (residual.dtype == (F32 if f32 else BF16) and residual.is_contiguous())
     y = torch.empty((N, D, H, W, Cout), device=x.device, dtype=F32 if out_f32 else BF16)
     g = _geom(N, D, H, W, Cin, Cout, k)
-    flags = (_lib.EPI_RELU if relu else 0) | (_lib.EPI_OUT_F32 if out_f32 else 0) | \
-        (_lib.EPI_RES_F32 if (f32 and residual is not None) else 0) | (_lib.EPI_IN_F32 if ffma else 0)
-    if ffma:
-        algo = _lib.ALGO_SIMT
+    flags = (_lib.EPI_RELU if relu else 0) | (_lib.EPI_OUT_F32 if out_f32 else 0) | (_lib.EPI_IN_F32 if f32 else 0)
     check(lib().t2v_conv_fprop(ctypes.byref(g), ptr(x), ptr(w), ptr(bias), ptr(residual), ptr(y), flags, algo,
                                stream()), "t2v_conv_fprop")
     return y
@@ -168,42 +135,31 @@ def conv_fprop_skip(x, w, bias, x2, w2, k=(3, 3, 3), relu=False):
 def conv_dgrad(dy, wT, k=(3, 3, 3), residual=None, relu=False, out_f32=False, algo=0, relu_ref=None):
     """dy (N,D,H,W,Cout) bf16, wT (Cin,taps,Cout) bf16 (from pack_dgrad_weight) -> dx (N,D,H,W,Cin).
     relu_ref (dx-shaped): dx is zeroed where relu_ref <= 0 (the ReLU in front of the convolution, fused).
-    fp32 storage: dy fp32, wT (Cin,taps,T*Cout) -> dx fp32."""
+    fp32 storage: dy, wT fp32 -> dx fp32."""
     require_cuda(dy, wT, residual, relu_ref)
-    f32 = dy.dtype == F32
+    f32 = dy.dtype == F32                         # fp32 parity mode on exact fp32 FMAs
     if relu_ref is not None:
         assert residual is None and relu_ref.is_contiguous() and relu_ref.dtype == dy.dtype
         assert tuple(relu_ref.shape) == tuple(dy.shape[:4]) + (wT.shape[0],)
         residual = relu_ref
     N, D, H, W, Cout = dy.shape
     Cin = wT.shape[0]
-    ffma = f32 and wT.dtype == F32
-    if ffma:
-        out_f32 = True
-    elif f32:
-        assert wT.shape[2] == SPLIT_TERMS * Cout
-        dy = split3(dy, 0)
-        Cout, out_f32 = SPLIT_TERMS * Cout, True
-    assert wT.shape[2] == Cout and dy.is_contiguous() and wT.is_contiguous() and (ffma or dy.dtype == BF16)
+    if f32:
+        out_f32, algo = True, _lib.ALGO_SIMT
+    assert wT.shape[2] == Cout and dy.is_contiguous() and wT.is_contiguous() and wT.dtype == dy.dtype
     dx = torch.empty((N, D, H, W, Cin), device=dy.device, dtype=F32 if out_f32 else BF16)
     g = _geom(N, D, H, W, Cin, Cout, k)
     flags = (_lib.EPI_RELU if relu else 0) | (_lib.EPI_OUT_F32 if out_f32 else 0) | \
-        (_lib.EPI_RELU_MASK if relu_ref is not None else 0) | (_lib.EPI_RES_F32 if (f32 and residual is not None) else 0) | \
-        (_lib.EPI_IN_F32 if ffma else 0)
-    if ffma:
-        algo = _lib.ALGO_SIMT
+        (_lib.EPI_RELU_MASK if relu_ref is not None else 0) | (_lib.EPI_IN_F32 if f32 else 0)
     check(lib().t2v_conv_dgrad(ctypes.byref(g), ptr(dy), ptr(wT), ptr(residual), ptr(dx), flags, algo, stream()),
           "t2v_conv_dgrad")
     return dx
 
 
-PAIRED_WGRAD = os.environ.get("T2V_PAIRED_WGRAD", "1") == "1"
-
-
 def conv_wgrad(dy, x, k=(3, 3, 3), out=None, accumulate=False, algo=0):
     """dw (Cout,taps,Cin) fp32 = sum_pos dy[pos,co] x[pos+tap,ci]."""
     require_cuda(dy, x)
-    if dy.dtype == F32 and FP32_ENGINE == "ffma":
+    if dy.dtype == F32:
         assert x.dtype == F32 and dy.is_contiguous() and x.is_contiguous() and x.shape[:4] == dy.shape[:4]
         N, D, H, W, Cout = dy.shape
         Cin = x.shape[-1]
@@ -215,12 +171,9 @@ def conv_wgrad(dy, x, k=(3, 3, 3), out=None, accumulate=False, algo=0):
         check(lib().t2v_conv_wgrad(ctypes.byref(g), ptr(dy), ptr(x), ptr(out), 1 if accumulate else 0,
                                    _lib.ALGO_SIMT_F32, stream()), "t2v_conv_wgrad")
         return out
-    if dy.dtype == F32:
-        assert x.dtype == F32
-        dy, x = split3(dy, 1), split3(x, 2)          # sum over T*N "samples" = the part products
     N, D, H, W, Cout = dy.shape
     Cin = x.shape[-1]
-    if (PAIRED_WGRAD and algo == 0 and tuple(k) == (1, 3, 3) and D == 1 and Cin == 32 and Cout in (16, 32)
+    if (algo == 0 and tuple(k) == (1, 3, 3) and D == 1 and Cin == 32 and Cout in (16, 32)
             and W % 2 == 0 and W >= 16 and H >= 4 and dy.is_contiguous() and x.is_contiguous()):
         # 32-channel rows are 64 bytes: TMA and the MMA tiles run half empty.  Pair adjacent w voxels (a free view):
         # 64-channel rows on the halo-resident kernel, then fold the pair products into the 3 real w taps.
@@ -366,54 +319,33 @@ def _pack_dgrad_bf16(w, CoutP, CinP):
     return wT
 
 
-def _parts(w):
-    """fp32 weight -> its bf16 parts a, b, c as fp32 tensors (w = a + b + c; once per weight version: tiny tensors)"""
-    a = cast_f32(cast_bf16(w))
-    r1 = (w - a).contiguous()
-    b = cast_f32(cast_bf16(r1))
-    return a, b, (r1 - b).contiguous()
-
-
-def _weight_segments(w, pack):
-    a, b, c = _parts(w)
-    pa, pb = pack(a), pack(b)
-    if SPLIT_TERMS == 3:
-        return torch.cat((pa, pa, pb), dim=2).contiguous()
-    pc = pack(c)
-    return torch.cat((pa, pa, pb, pa, pc, pb), dim=2).contiguous()
-
-
 def pack_weight(w, CoutP=None, CinP=None):
     """w (Cout,taps,Cin) fp32 -> bf16 (CoutP,taps,CinP), zero padded (plain cast when unpadded).
-    fp32 storage mode: (CoutP,taps,T*CinP), the weight-side part order of t2v_split_bf16 along K."""
+    fp32 storage mode: fp32 (CoutP,taps,CinP)."""
     require_cuda(w)
     assert w.dtype == F32 and w.is_contiguous() and w.dim() == 3
     Cout, taps, Cin = w.shape
     CoutP, CinP = CoutP or Cout, CinP or Cin
-    if STORE == F32 and FP32_ENGINE == "ffma":
+    if STORE == F32:
         if (CoutP, CinP) == (Cout, Cin):
             return w.clone()
         wp = torch.zeros((CoutP, taps, CinP), device=w.device, dtype=F32)
         wp[:Cout, :, :Cin] = w
         return wp
-    if STORE == F32:
-        return _weight_segments(w, lambda t: _pack_weight_bf16(t, CoutP, CinP))
     return _pack_weight_bf16(w, CoutP, CinP)
 
 
 def pack_dgrad_weight(w, CoutP=None, CinP=None):
     """w (Cout,taps,Cin) fp32 -> (CinP,taps,CoutP) bf16 with the tap order reversed
-    (fp32 storage mode: (CinP,taps,T*CoutP), weight-side part order)."""
+    (fp32 storage mode: fp32 (CinP,taps,CoutP))."""
     require_cuda(w)
     assert w.dtype == F32 and w.is_contiguous() and w.dim() == 3
     Cout, taps, Cin = w.shape
     CoutP, CinP = CoutP or Cout, CinP or Cin
-    if STORE == F32 and FP32_ENGINE == "ffma":
+    if STORE == F32:
         wp = torch.zeros((CinP, taps, CoutP), device=w.device, dtype=F32)
         wp[:Cin, :, :Cout] = w.flip(1).permute(2, 1, 0)           # tap order reversed, channels transposed
         return wp
-    if STORE == F32:
-        return _weight_segments(w, lambda t: _pack_dgrad_bf16(t, CoutP, CinP))
     return _pack_dgrad_bf16(w, CoutP, CinP)
 
 
@@ -448,7 +380,7 @@ def gconv_pack(w3):
 
 
 # --- kernel-4 / stride-2 / padding-1 layers on the tcgen05 engine (csrc/s2d.cu: shifted space-to-depth blocks) --------
-GCONV_TC = os.environ.get("T2V_GCONV_TC", "1") == "1"
+GCONV_TC = True          # False: every general convolution on the CUDA-core kernels (the reference of the tests)
 
 
 def round16(c):
@@ -1177,17 +1109,6 @@ def adam_step(params, grads, ms, vs, lr, beta1, beta2, eps, step, grad_scale=1.0
     check(lib().t2v_adam_step(n, arr(*[p.data_ptr() for p in params]), arr(*[g.data_ptr() for g in grads]),
                               arr(*[m.data_ptr() for m in ms]), arr(*[v.data_ptr() for v in vs]), sizes, lr, beta1,
                               beta2, eps, step, grad_scale, ptr(dyn), stream()), "t2v_adam_step")
-
-
-def stream_copy(src, dst, ctas=32):
-    """dst <- src (same byte size, contiguous), by `ctas` resident CTAs; src may be pinned host memory."""
-    if not ((src.is_cuda or src.is_pinned()) and dst.is_cuda):
-        raise _lib.T2VError("stream_copy needs a CUDA or pinned source and a CUDA destination")
-    nbytes = src.numel() * src.element_size()
-    assert nbytes == dst.numel() * dst.element_size() and src.is_contiguous() and dst.is_contiguous()
-    assert nbytes % 16 == 0 and src.data_ptr() % 16 == 0 and dst.data_ptr() % 16 == 0
-    check(lib().t2v_stream_copy(ptr(src), ptr(dst), nbytes, ctas, stream()), "t2v_stream_copy")
-    return dst
 
 
 def multi_copy(srcs, dsts):

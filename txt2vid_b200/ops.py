@@ -10,7 +10,6 @@ fp32 `nn.Parameter`s with the reference's logical shapes; conv weights are re-ho
 channels-last memory ([Cout][taps][Cin]) so that packing is a cast and the weight gradient the
 kernels write is the parameter gradient's memory.
 """
-import os
 import weakref
 
 import torch
@@ -168,7 +167,6 @@ PACKS = _PackCache()
 # iteration.  Instead every unpadded conv weight owns one persistent fp32 buffer [Cout][taps][Cin] (= p.grad's memory,
 # zeroed by zero_grads) and the weight-gradient kernels accumulate into it directly (fp32 red.add, as they already
 # do between their own position splits).  Second-order graphs (create_graph=True) keep the functional path.
-GRAD_SINKS = os.environ.get("T2V_GRAD_SINKS", "1") == "1"
 
 
 def _sinkable(p):
@@ -198,14 +196,14 @@ def zero_grads(module):
         mark_conv_weights(module)
     bufs = []
     for p in module.parameters():
-        if GRAD_SINKS and p.requires_grad and getattr(p, "_t2v_bias", False) and p.dim() == 1 and p.numel() % 16 == 0:
+        if p.requires_grad and getattr(p, "_t2v_bias", False) and p.dim() == 1 and p.numel() % 16 == 0:
             # conv biases: the column-sum kernel adds into the gradient buffer (t2v_sum_rows_acc)
             if p.grad is None or not getattr(p, "_t2v_bias_sink", False):
                 p.grad = torch.empty_like(p)
                 p._t2v_bias_sink = True
             bufs.append(p.grad)
             continue
-        if not (GRAD_SINKS and p.requires_grad and _sinkable(p)):
+        if not (p.requires_grad and _sinkable(p)):
             p.grad = None
             continue
         w3 = w3_view(p)                                  # re-homes the parameter to channels-last memory if needed
@@ -262,7 +260,6 @@ def _pad_bias(bias, CoutP):
 
 
 # ------------------------------------------------------------------------------------- convolution
-FUSE_RELU_BWD = os.environ.get("T2V_FUSE_RELU_BWD", "1") == "1"
 
 
 class ConvF(Function):
@@ -374,7 +371,7 @@ class ConvSkipF(Function):
 
 
 def conv_skip(h, x, weight, bias, wskip, bskip, h_relu=False):
-    return ConvSkipF.apply(h, x, weight, bias, wskip, bskip, h_relu and FUSE_RELU_BWD)
+    return ConvSkipF.apply(h, x, weight, bias, wskip, bskip, h_relu)
 
 
 class ConvDgradF(Function):
@@ -494,7 +491,7 @@ class ConvSd2WgradF(Function):
 
 
 def conv_sd2(x, weight, bias=None, x_relu=False):
-    return ConvSd2F.apply(x, weight, bias, x_relu and FUSE_RELU_BWD)
+    return ConvSd2F.apply(x, weight, bias, x_relu)
 
 
 class SumRowsF(Function):
@@ -514,7 +511,7 @@ class SumRowsF(Function):
 
 def conv(x, weight, bias=None, residual=None, relu=False, x_relu=False, relu_later=False):
     """x_relu / relu_later: see ConvF (both must be set consistently by the block that wires producer and consumer)."""
-    return ConvF.apply(x, weight, bias, residual, relu, x_relu and FUSE_RELU_BWD, relu_later and FUSE_RELU_BWD)
+    return ConvF.apply(x, weight, bias, residual, relu, x_relu, relu_later)
 
 
 # ------------------------------------------------------------------------------------- general conv (TGAN / TCWYT)
@@ -744,7 +741,7 @@ class ReluBwdF(Function):
 
 def relu(x, later=False):
     """later=True: the consumers apply the backward mask (ops.conv(..., x_relu=True))."""
-    return ReluF.apply(x, later and FUSE_RELU_BWD)
+    return ReluF.apply(x, later)
 
 
 # ------------------------------------------------------------------------------------- avg-pool
@@ -942,15 +939,13 @@ class StemConvF(Function):
         ctx.bias_ref = bias
         ctx.x_leaf = x.is_leaf
         y = K.stem_fprop(xc, _stem_pack(weight), None if bias is None else bias.detach(), True)
-        ctx.save_for_backward(xc, weight, None if FUSE_RELU_BWD else y)
+        ctx.save_for_backward(xc, weight)
         return y
 
     @staticmethod
     def backward(ctx, dy):
-        xc, weight, y = ctx.saved_tensors
+        xc, weight = ctx.saved_tensors
         dy = dy.contiguous()
-        if y is not None:                    # T2V_FUSE_RELU_BWD=0: no consumer applies this op's ReLU mask
-            dy = ReluBwdF.apply(dy, y)
         dx = dw = db = None
         if ctx.needs_input_grad[0] and not (ctx.x_leaf and _SKIP_LEAF_INPUT_GRADS[0] and not torch.is_grad_enabled()):
             w2d = stem_weight_2d(weight)
@@ -1093,7 +1088,6 @@ def gather_frames(x, B, T, bt):
 
 
 # ------------------------------------------------------------------------------------- ConvLSTM
-LSTM_FUSED = os.environ.get("T2V_LSTM_FUSED", "1") == "1"
 
 
 class ConvLstmF(Function):
@@ -1113,7 +1107,7 @@ class ConvLstmF(Function):
         k = (1, 3, 3) if taps == 9 else (1, 1, 1)
         gates, cs, hs = [], [], []
         h = c = None
-        if LSTM_FUSED and not fp32_mode() and hasattr(K, "conv_lstm_step") and Hd % 32 == 0 and x.shape[-1] % 16 == 0:
+        if not fp32_mode() and hasattr(K, "conv_lstm_step") and Hd % 32 == 0 and x.shape[-1] % 16 == 0:
             # gate GEMM + sigmoid / tanh cell update in ONE kernel per step (t2v_conv_lstm_step): the gates are
             # interleaved per 32 hidden units along Cout so that an accumulator tile carries [i|f|g|o] of its units;
             # h_t goes to the next step's operand AND to its (b, t) slot of the merged frame map from the epilogue

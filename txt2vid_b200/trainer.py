@@ -205,10 +205,10 @@ def hostrng_ring():
 
 
 class GraphedTrainStep(object):
-    """The training iteration as three replayed CUDA graphs (no tracing compiler: the eager iteration above is
-    captured as is).  Segments: [pyramid, G fwd, D fwd/bwd incl. gradient penalty] -> (all-reduce D grads) ->
-    [Adam D, real_pred, G-step fwd/bwd] -> (all-reduce G grads) -> [Adam G].  Everything the host decides per
-    iteration reaches the kernels through device buffers refreshed before each replay: the batch, the caption
+    """The training iteration as ONE replayed CUDA graph (no tracing compiler: the eager iteration above is
+    captured as is): pyramid, G fwd, D fwd/bwd incl. gradient penalty, all-reduce of the D grads, Adam D,
+    real_pred, G-step fwd/bwd, all-reduce of the G grads, Adam G.  `graphs` is the 1-tuple of that graph.
+    Everything the host decides per iteration reaches the kernels through device buffers refreshed before each replay: the batch, the caption
     embedding (the Bi-LSTM runs eagerly -- variable lengths), the host-RNG draws (hostrng.StaticDraws, same
     generators and order as the reference), Adam's bias corrections.  z comes from the CUDA generator inside
     the graph.  Needs discrim_steps = gen_steps = 1, a fixed batch shape and an even frame count per level."""
@@ -223,8 +223,6 @@ class GraphedTrainStep(object):
         self.side = torch.cuda.Stream(device=device)
         # per-replay host values (RNG draws, Adam bias corrections) go through a ring of pinned staging slots: the
         # H2D copies are asynchronous, so a slot is rewritten only after the copies issued from it have executed
-        import os
-        self.single_graph = os.environ.get("T2V_SINGLE_GRAPH", "1") == "1"
         self.ring = hostrng_ring()
         self.stage_evt = [None] * self.ring
         self.replays = 0
@@ -250,36 +248,23 @@ class GraphedTrainStep(object):
         torch.cuda.synchronize()
         pool = torch.cuda.graph_pool_handle()
         self.draws.begin_iteration()
-        if self.single_graph:
-            # ONE graph for the whole iteration; the two NCCL all-reduces are captured with it (thread-local capture
-            # mode: NCCL's watchdog thread may touch the CUDA API meanwhile).  Separate graphs with eager all-reduces
-            # between them leave cross-stream waits in front of each replay: measured at two GPUs the step then
-            # flips between 90 and 130 ms.
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g, pool=pool, stream=self.side, capture_error_mode="thread_local"):
-                st = _d_phase(self.gan, self.static_x, self.static_cond, dev, self.params, self.losses, None,
-                              self.channel_first, False)
-                if self.dist is not None:
-                    self.dist.reduce_grads(self.optD)
-                self.optD.step()
-                st = _g_phase(self.gan, st, self.params, self.losses)
-                if self.dist is not None:
-                    self.dist.reduce_grads(self.optG)
-                self.optG.step()
-            self.state = st
-            self.graphs = (g,)
-            return
-        g1, g2, g3 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g1, pool=pool, stream=self.side):
+        # ONE graph for the whole iteration; the two NCCL all-reduces are captured with it (thread-local capture
+        # mode: NCCL's watchdog thread may touch the CUDA API meanwhile).  Separate graphs with eager all-reduces
+        # between them leave cross-stream waits in front of each replay: measured at two GPUs the step then
+        # flips between 90 and 130 ms.
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, pool=pool, stream=self.side, capture_error_mode="thread_local"):
             st = _d_phase(self.gan, self.static_x, self.static_cond, dev, self.params, self.losses, None,
                           self.channel_first, False)
-        with torch.cuda.graph(g2, pool=pool, stream=self.side):
+            if self.dist is not None:
+                self.dist.reduce_grads(self.optD)
             self.optD.step()
             st = _g_phase(self.gan, st, self.params, self.losses)
-        with torch.cuda.graph(g3, pool=pool, stream=self.side):
+            if self.dist is not None:
+                self.dist.reduce_grads(self.optG)
             self.optG.step()
         self.state = st
-        self.graphs = (g1, g2, g3)
+        self.graphs = (g,)
 
     def __call__(self, x, y):
         """x (B,T,C,H,W) on the device (or pinned host), y = [tokens, lengths] -> (lossD, lossG) device scalars."""
@@ -331,17 +316,7 @@ class GraphedTrainStep(object):
         self._stage_adam(self.optG, self.optG._step_count + 1, slot)
         self.stage_evt[slot] = torch.cuda.Event()
         self.stage_evt[slot].record()
-        if len(self.graphs) == 1:
-            self.graphs[0].replay()
-        else:
-            g1, g2, g3 = self.graphs
-            g1.replay()
-            if self.dist is not None:
-                self.dist.reduce_grads(self.optD)
-            g2.replay()
-            if self.dist is not None:
-                self.dist.reduce_grads(self.optG)
-            g3.replay()
+        self.graphs[0].replay()
         for opt in (self.optD, self.optG):
             opt._step_count += 1
         ops.bump_weight_epoch()          # eager users of the modules must re-pack the updated weights
