@@ -32,6 +32,20 @@ def test_no_cpu_fallback():
                      k=(1, 1, 1))
 
 
+def test_channel_reductions_reject_channel_counts_not_multiple_of_8():
+    """the column reductions read 8 channels per load: C % 8 != 0 is refused before any CUDA call"""
+    from txt2vid_b200 import _lib
+    lib = _lib.lib()
+    ERR_ARG = -1                                      # T2V_ERR_ARG of include/t2v.h
+    for sfx in ("", "_f32"):
+        assert getattr(lib, "t2v_sum_rows" + sfx)(None, None, 5, 12, None) == ERR_ARG
+        assert getattr(lib, "t2v_sum_rows_acc" + sfx)(None, None, 5, 12, None) == ERR_ARG
+        assert getattr(lib, "t2v_sum_spatial" + sfx)(None, None, 2, 3, 12, None) == ERR_ARG
+        assert getattr(lib, "t2v_bn_stats" + sfx)(None, None, 5, 12, None) == ERR_ARG
+        assert getattr(lib, "t2v_bn_bwd" + sfx)(None, None, None, None, None, None, 1, 1, 5, 12, 0, 1,
+                                               None) == ERR_ARG
+
+
 def test_environment_reads_are_diagnostics_and_launcher_variables_only():
     """The product reads no environment variable that selects a code path or a tuning value: what runs depends on
     the inputs and the code only.  Allowed are the diagnostics T2V_PROFILE_DUMP / T2V_DEBUG_LAUNCH (they print,

@@ -98,9 +98,10 @@ def test_layout_roundtrip():
     assert torch.equal(K().cl_to_nchw(y, 3), C.cl_to_nchw(y, 3))
 
 
-@pytest.mark.parametrize("Cc", [16, 64, 96, 256, 1024, 40])
+@pytest.mark.parametrize("Cc", [16, 64, 96, 256, 1024, 40, 24, 48, 368, 1000])
 def test_sum_rows_paths(Cc):
-    """vectorised column reduction (C/8 a power of two, 256-channel slabs) and the scalar fallback"""
+    """vectorised column reduction: C/8 a power of two (every thread reads rows), C/8 not dividing 256 (idle threads
+    past the last row slot), 256-channel slabs with a narrower last slab"""
     x = rnd(37, 1, 3, 5, Cc)
     close(K().sum_rows(x), C.sum_rows(x), 1e-3)
     x = rnd(5000, 1, 1, 1, Cc)
@@ -113,6 +114,17 @@ def test_reductions():
     close(K().sum_spatial(x), C.sum_spatial(x), 1e-3)
     g = torch.randn(7, 96, device="cuda")
     assert torch.equal(K().broadcast_spatial(g, x.shape), C.broadcast_spatial(g, x.shape))
+    x = rnd(70000, 1, 1, 2, 16)                      # more samples than a grid.y / grid.z dimension holds
+    close(K().sum_spatial(x), C.sum_spatial(x), 1e-3)
+
+
+@pytest.mark.parametrize("dt", [BF, torch.float32])
+@pytest.mark.parametrize("S", [1, 16, 300])
+@pytest.mark.parametrize("Cc", [96, 368, 1024])
+def test_sum_spatial_paths(Cc, S, dt):
+    """per-sample spatial sum (one block row per sample) in both storage types"""
+    x = rnd(5, 1, 1, S, Cc, dtype=dt)
+    close(K().sum_spatial(x), C.sum_spatial(x), 1e-4)
 
 
 def test_activations():
@@ -154,7 +166,8 @@ def test_gconv(case):
     close(K().gconv_wgrad(dy, x, k, s, p), C.gconv_wgrad(dy, x, k, s, p), 2e-3)
 
 
-@pytest.mark.parametrize("Cc,shape", [(64, (6, 1, 8, 8)), (512, (4, 2, 3, 3)), (1024, (16, 1, 2, 2)), (48, (5, 1, 4, 4))])
+@pytest.mark.parametrize("Cc,shape", [(64, (6, 1, 8, 8)), (512, (4, 2, 3, 3)), (1024, (16, 1, 2, 2)), (48, (5, 1, 4, 4)),
+                                      (368, (50, 1, 2, 3))])
 @pytest.mark.parametrize("act", [0, 1, 2])
 def test_batchnorm_any_shape(Cc, shape, act):
     """BatchNorm1d/2d/3d statistics over all leading dims + fused activation codes (0 none, 1 ReLU, 2 LeakyReLU)"""

@@ -86,6 +86,21 @@ def test_fp32_storage_kernels_match_spec(precision):
     assert torch.equal(K().f32_pad_cl(sl, 32, dt)[..., :20].float(), sl.to(dt).float())
 
 
+@pytest.mark.parametrize("Cc", [48, 368])
+def test_fp32_batchnorm_statistics_are_bit_reproducible(Cc):
+    """fp32 storage: BatchNorm statistics are reduced in a fixed order for every channel count, so two runs on the same
+    input agree bit for bit (C = 48: C/8 does not divide 256; C = 368: a narrower second 256-channel slab)"""
+    x = torch.randn(20000, 1, 1, 1, Cc, device="cuda", generator=torch.Generator(device="cuda").manual_seed(1)) + 0.5
+    gamma, beta = torch.rand(Cc, device="cuda") + 0.5, torch.randn(Cc, device="cuda")
+    runs = []
+    for _ in range(2):
+        rm, rv = torch.zeros(Cc, device="cuda"), torch.ones(Cc, device="cuda")
+        y, mi, ss = K().bn_forward(x, gamma, beta, rm, rv, 1, 1)
+        runs.append((y, mi, ss, rm, rv))
+    for a, b in zip(*runs):
+        assert torch.equal(a, b)
+
+
 @pytest.mark.parametrize("epilogue", ["residual", "relu"])
 @pytest.mark.parametrize("geom", [((4, 1, 8, 8), 64, 64, (1, 3, 3)), ((2, 4, 4, 4), 128, 64, (3, 3, 3)),
                                   ((16, 1, 1, 1), 256, 512, (1, 1, 1)), ((2, 2, 8, 8), 16, 32, (3, 3, 3)),
