@@ -275,6 +275,15 @@ int t2v_bn_apply(const void* x, const float* scale_shift, void* y, int64_t N, in
 /* red fp32 [2C] = {dbeta, dgamma}; dx (N,H,W,C)                                                   */
 int t2v_bn_bwd(const void* dy, const void* x, const float* scale_shift, const float* mean_invstd, float* red,
                void* dx, int64_t N, int32_t H, int32_t W, int32_t C, int32_t relu, int32_t up, void* stream);
+/* double backward of t2v_bn_bwd (up == 1) seen as (dy, x, gamma) -> (dx, dgamma, dbeta), for second-order graphs
+ * (the critics' gradient penalty).  x, dy (P,C) CL with the same scale_shift / mean_invstd; upstream gradients
+ * ggx (P,C) w.r.t. dx and ggamma / ggbeta fp32 [C] w.r.t. dgamma / dbeta (NULL = zero).  Writes gx (P,C), the
+ * gradient w.r.t. x; gdy (P,C), the gradient w.r.t. dy (activation mask applied, as in t2v_bn_bwd); dgamma_out fp32
+ * [C], the gradient w.r.t. gamma; red fp32 [5C] receives the per-channel sums {g, g*xhat, ggx, ggx*xhat, ggx*g}
+ * (g = masked dy).  Float atomics, no scratch allocation.  T2V_ERR_ARG for up != 1 or C % 8 != 0.            */
+int t2v_bn_bwd_bwd(const void* dy, const void* x, const void* ggx, const float* ggamma, const float* ggbeta,
+                   const float* scale_shift, const float* mean_invstd, float* red, void* gx, void* gdy,
+                   float* dgamma_out, int64_t P, int32_t C, int32_t relu, int32_t up, void* stream);
 
 /* Fused core of the non-local block (models/layers.py:23-36,52-68): o = softmax(theta . maxpool(phi)^T) . maxpool(g)
  * per map, max-pool (1,2,2); theta/phi (N,D,H,W,C8p) and g/o (N,D,H,W,C2p) bf16 CL with c8 <= 8, c2 <= 16 real
@@ -362,6 +371,9 @@ int t2v_bn_apply_f32(const void* x, const float* scale_shift, void* y, int64_t N
                      int32_t relu, int32_t up, void* stream);
 int t2v_bn_bwd_f32(const void* dy, const void* x, const float* scale_shift, const float* mean_invstd, float* red,
                    void* dx, int64_t N, int32_t H, int32_t W, int32_t C, int32_t relu, int32_t up, void* stream);
+int t2v_bn_bwd_bwd_f32(const void* dy, const void* x, const void* ggx, const float* ggamma, const float* ggbeta,
+                       const float* scale_shift, const float* mean_invstd, float* red, void* gx, void* gdy,
+                       float* dgamma_out, int64_t P, int32_t C, int32_t relu, int32_t up, void* stream);
 int t2v_render_fwd_f32(const void* pre, float* y, int32_t B, int32_t T, int32_t H, int32_t W, int32_t C, int32_t Cp,
                        void* stream);
 int t2v_render_bwd_f32(const float* dy, const float* y, void* dpre, int32_t B, int32_t T, int32_t H, int32_t W,

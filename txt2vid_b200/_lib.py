@@ -118,6 +118,7 @@ SIGNATURES = {
     "t2v_bn_finalize": [_P, _P, _P, _P, _P, _P, _P, c_i32, c_i64, c_float, c_float, _P],
     "t2v_bn_apply": [_P, _P, _P, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, _P],
     "t2v_bn_bwd": [_P, _P, _P, _P, _P, _P, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, _P],
+    "t2v_bn_bwd_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_i64, c_i32, c_i32, c_i32, _P],
     "t2v_attention_fwd": [_P, _P, _P, _P, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, _P],
     "t2v_attention_bwd": [_P, _P, _P, _P, _P, _P, _P, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, _P],
     "t2v_attention_bwd_large": [_P, _P, _P, _P, _P, _P, _P, _P, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32,
@@ -137,7 +138,8 @@ SIGNATURES = {
 _TYPED = ["t2v_relu_fwd", "t2v_relu_bwd", "t2v_leaky_relu_fwd", "t2v_leaky_relu_bwd", "t2v_tanh_fwd", "t2v_tanh_bwd",
           "t2v_avgpool_fwd", "t2v_avgpool_bwd", "t2v_upsample2x_fwd", "t2v_upsample2x_bwd", "t2v_nchw_to_cl",
           "t2v_cl_to_nchw", "t2v_im2col3", "t2v_col2im3", "t2v_sum_rows", "t2v_sum_rows_acc", "t2v_sum_spatial",
-          "t2v_broadcast_spatial", "t2v_bn_stats", "t2v_bn_apply", "t2v_bn_bwd", "t2v_render_fwd", "t2v_render_bwd",
+          "t2v_broadcast_spatial", "t2v_bn_stats", "t2v_bn_apply", "t2v_bn_bwd", "t2v_bn_bwd_bwd", "t2v_render_fwd",
+          "t2v_render_bwd",
           "t2v_lstm_cell_fwd", "t2v_lstm_cell_bwd", "t2v_gconv_fprop", "t2v_gconv_dgrad", "t2v_gconv_wgrad",
           "t2v_scale", "t2v_scale_add", "t2v_dot", "t2v_cl_slice_f32", "t2v_f32_pad_cl", "t2v_lstm_seq_fwd",
           "t2v_lstm_seq_bwd", "t2v_embedding_fwd", "t2v_embedding_bwd"]

@@ -138,7 +138,9 @@ def fused_loss_mode(loss, which):
 def _gradient_penalty(discrim, real_x=None, real_xbar=None, fake_x=None, fake_xbar=None, real_cond=None,
                       fake_cond=None, zero_center=False, combine=torch.mean):
     """gan/losses.py:135-186.  alpha ~ U(0,1) per sample from the CPU generator (created on CPU, then moved,
-    :140-145); only d/dx_hat is kept (:178); the second derivative runs through ops.Conv*F etc."""
+    :140-145); only d/dx_hat is kept (:178); the second derivative runs through ops.Conv*F etc.  A critic that
+    returns one tensor instead of the (uncond, cond, features) tuple (TGAN / TCWYT VideoDiscrim: the scalar mean
+    of its output map) has that tensor as its only output."""
     B = real_x.size(0)
     assert real_x.dim() in (4, 5)
     alpha = hostrng.CURRENT.alpha(B, real_x.device)            # B draws from the CPU generator, as the reference
@@ -155,8 +157,12 @@ def _gradient_penalty(discrim, real_x=None, real_xbar=None, fake_x=None, fake_xb
     ch = None
     if real_cond is not None and fake_cond is not None:
         ch = lerp(real_cond, fake_cond)
-    u, c, _ = discrim(x=xh, cond=ch, xbar=xbarh)
-    outs = [u] + ([c] if c is not None else [])
+    out = discrim(x=xh, cond=ch, xbar=xbarh)
+    if isinstance(out, torch.Tensor):
+        outs = [out]
+    else:
+        u, c, _ = out
+        outs = [u] + ([c] if c is not None else [])
     ins = [xh] + ([ch] if ch is not None else []) + ([xbarh] if xbarh is not None else [])
     g = torch.autograd.grad(outputs=outs, inputs=ins, grad_outputs=[torch.ones_like(o) for o in outs],
                             create_graph=True, retain_graph=True, only_inputs=True)[0]

@@ -953,6 +953,27 @@ def bn_backward(dy, x, mean_invstd, scale_shift, relu, up):
     return dx.view(shape0), red[C:], red[:C]
 
 
+def bn_backward_backward(dy, x, mean_invstd, scale_shift, ggx, ggamma, ggbeta, relu, up):
+    """Double backward of bn_backward (up == 1): upstream ggx (x-shaped CL, w.r.t. dx) and ggamma / ggbeta (fp32 [C]
+    w.r.t. dgamma / dbeta, None = zero) -> gx (w.r.t. x), gdy (w.r.t. dy), both x-shaped CL, and dgamma fp32 [C]
+    (w.r.t. gamma)."""
+    require_cuda(dy, x, ggx, ggamma, ggbeta)
+    _act(dy, x, ggx)
+    assert up == 1, "the double backward has no upsampling form"
+    C = x.shape[-1]
+    P = x.numel() // C
+    assert dy.dtype == x.dtype == ggx.dtype and dy.numel() == ggx.numel() == x.numel()
+    for t in (ggamma, ggbeta):
+        assert t is None or (t.dtype == F32 and t.is_contiguous() and t.numel() == C)
+    red = torch.empty((5 * C,), device=x.device, dtype=F32)
+    gx, gdy = torch.empty_like(x), torch.empty_like(x)
+    dgamma = torch.empty((C,), device=x.device, dtype=F32)
+    check(_lib.typed("t2v_bn_bwd_bwd", x)(ptr(dy), ptr(x), ptr(ggx), ptr(ggamma), ptr(ggbeta), ptr(scale_shift),
+                                          ptr(mean_invstd), ptr(red), ptr(gx), ptr(gdy), ptr(dgamma), P, C, int(relu),
+                                          up, stream()), "t2v_bn_bwd_bwd")
+    return gx, gdy, dgamma
+
+
 # ------------------------------------------------------------------------------------- non-local attention core
 def attention_fwd(theta, phi, g, c8, c2):
     """theta/phi (N,D,H,W,C8p), g (N,D,H,W,C2p) bf16 -> o (N,D,H,W,C2p): softmax(theta . maxpool(phi)^T) . maxpool(g)."""

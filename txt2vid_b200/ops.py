@@ -530,8 +530,9 @@ def conv_args(module):
 
 
 class GConvF(Function):
-    """Strided / padded convolution on a CL tensor (first-order): the k4 s2 p1 and head convolutions of
-    models/tcwyt/video_discrim.py:12-46, frame_discrim.py:8-49, motion_discrim.py:8-19."""
+    """Strided / padded convolution on a CL tensor: the k4 s2 p1 and head convolutions of
+    models/tcwyt/video_discrim.py:12-46, frame_discrim.py:8-49, motion_discrim.py:8-19.  The backward is composed of
+    GConvDgradF / GConvWgradF, so the critics' gradient penalty can differentiate it a second time."""
 
     @staticmethod
     def forward(ctx, x, weight, bias, k, s, p, out_f32=False):
@@ -544,24 +545,59 @@ class GConvF(Function):
         return y
 
     @staticmethod
-    @once_differentiable
     def backward(ctx, dy):
         k, s, p, has_bias = ctx.cfg
         x, weight = ctx.saved_tensors
         dy = dy.contiguous()
         if dy.dtype != x.dtype:                      # fp32 output of a critic's last layer in bf16 storage mode
-            dy = K.cast_bf16(dy)
-        Cout, Cin = weight.shape[0], weight.shape[1]
+            dy = CastStoreF.apply(dy)
         dx = dw = db = None
         if ctx.needs_input_grad[0]:
-            wp = PACKS.get(weight, "gconv", dy.shape[-1], x.shape[-1])
-            dx = K.gconv_dgrad(dy, wp, None, tuple(x.shape[1:4]), k, s, p, cin_real=Cin)
+            dx = GConvDgradF.apply(dy, weight, tuple(x.shape[1:4]), x.shape[-1], k, s, p)
         if ctx.needs_input_grad[1]:
-            dw3 = K.unpack_wgrad(K.gconv_wgrad(dy, x, k, s, p, cin_real=Cin), Cout, Cin)
-            dw = grad_like_weight(dw3, weight)
+            dw = GConvWgradF.apply(dy, x, weight, k, s, p)
         if has_bias and ctx.needs_input_grad[2]:
-            db = K.sum_rows(dy)[:Cout]
+            db = SumRowsF.apply(dy)[:weight.shape[0]]
         return dx, dw, db, None, None, None, None
+
+
+class GConvDgradF(Function):
+    """dx = gconv_dgrad(dy, w): the data gradient of GConvF, itself differentiable (d/d(dy) = the convolution of the
+    upstream gradient, d/dw = the weight gradient of dy against it)."""
+
+    @staticmethod
+    def forward(ctx, dy, weight, in_sp, CinP, k, s, p):
+        wp = PACKS.get(weight, "gconv", dy.shape[-1], CinP)
+        ctx.cfg = (k, s, p)
+        ctx.save_for_backward(dy, weight)
+        return K.gconv_dgrad(dy, wp, None, in_sp, k, s, p, cin_real=weight.shape[1])
+
+    @staticmethod
+    def backward(ctx, ggx):
+        k, s, p = ctx.cfg
+        dy, weight = ctx.saved_tensors
+        ggx = ggx.contiguous()
+        g_dy = g_w = None
+        if ctx.needs_input_grad[0]:
+            g_dy = GConvF.apply(ggx, weight, None, k, s, p, False)
+        if ctx.needs_input_grad[1]:
+            g_w = GConvWgradF.apply(dy, ggx, weight, k, s, p)
+        return g_dy, g_w, None, None, None, None, None
+
+
+class GConvWgradF(Function):
+    """dw = gconv_wgrad(dy, x), returned with the parameter's logical shape."""
+
+    @staticmethod
+    def forward(ctx, dy, x, weight, k, s, p):
+        Cout, Cin = weight.shape[0], weight.shape[1]
+        dw3 = K.unpack_wgrad(K.gconv_wgrad(dy, x, k, s, p, cin_real=Cin), Cout, Cin)
+        return grad_like_weight(dw3, weight)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, ddw):
+        raise NotImplementedError("third-order graph through the general convolution's weight gradient")
 
 
 class GConvTF(Function):
@@ -615,7 +651,8 @@ def gconv_transpose(x, module, out_f32=False):
 
 
 class CastStoreF(Function):
-    """fp32 CL -> the storage dtype (bf16 mode: one rounding); backward: the gradient back in fp32"""
+    """fp32 CL -> the storage dtype (bf16 mode: one rounding); backward: the gradient back in fp32.  A cast is
+    linear, so each direction's backward is the other one (CastF32F) and second-order graphs pass through."""
 
     @staticmethod
     def forward(ctx, x):
@@ -623,7 +660,19 @@ class CastStoreF(Function):
 
     @staticmethod
     def backward(ctx, dy):
-        return K.cast_f32(dy.contiguous()) if dy.dtype == BF16 else dy
+        return CastF32F.apply(dy.contiguous()) if dy.dtype == BF16 else dy
+
+
+class CastF32F(Function):
+    """bf16 CL -> fp32 (the backward of CastStoreF); backward: the gradient rounded back to bf16"""
+
+    @staticmethod
+    def forward(ctx, x):
+        return K.cast_f32(x)
+
+    @staticmethod
+    def backward(ctx, g):
+        return CastStoreF.apply(g.contiguous())
 
 
 def conv_bn_act(x, conv_module, bn, act, transpose=False):
@@ -648,10 +697,24 @@ class LeakyF(Function):
         return y
 
     @staticmethod
-    @once_differentiable
     def backward(ctx, dy):
         (y,) = ctx.saved_tensors
-        return K.leaky_relu_bwd(dy.contiguous(), y, ctx.slope), None
+        return LeakyBwdF.apply(dy.contiguous(), y, ctx.slope), None
+
+
+class LeakyBwdF(Function):
+    """dx = dy * (ref > 0 ? 1 : slope); linear in dy, piecewise constant in ref (no gradient w.r.t. ref)."""
+
+    @staticmethod
+    def forward(ctx, dy, ref, slope):
+        ctx.slope = slope
+        ctx.save_for_backward(ref)
+        return K.leaky_relu_bwd(dy, ref, slope)
+
+    @staticmethod
+    def backward(ctx, ggx):
+        (ref,) = ctx.saved_tensors
+        return LeakyBwdF.apply(ggx.contiguous(), ref, ctx.slope), None, None
 
 
 def leaky_relu(x, slope=0.2):
@@ -1026,17 +1089,48 @@ class BnReluUpF(Function):
         y, mean_invstd, scale_shift = K.bn_forward(x, gamma.detach(), beta.detach(), running_mean, running_var, relu,
                                                    up, eps, momentum, training)
         ctx.cfg = (relu, up, training)
-        ctx.save_for_backward(x, mean_invstd, scale_shift)
+        ctx.save_for_backward(x, gamma, mean_invstd, scale_shift)
         return y
 
     @staticmethod
-    @once_differentiable
     def backward(ctx, dy):
         relu, up, training = ctx.cfg
-        x, mean_invstd, scale_shift = ctx.saved_tensors
+        x, gamma, mean_invstd, scale_shift = ctx.saved_tensors
         assert training, "eval-mode BatchNorm backward is not on the training path"
-        dx, dgamma, dbeta = K.bn_backward(dy.contiguous(), x, mean_invstd, scale_shift, relu, up)
+        if torch.is_grad_enabled():          # create_graph: the backward itself is differentiable (BnBwdF)
+            dx, dgamma, dbeta = BnBwdF.apply(dy.contiguous(), x, gamma, mean_invstd, scale_shift, relu, up)
+        else:
+            dx, dgamma, dbeta = K.bn_backward(dy.contiguous(), x, mean_invstd, scale_shift, relu, up)
         return dx, dgamma, dbeta, None, None, None, None, None, None, None
+
+
+class BnBwdF(Function):
+    """(dx, dgamma, dbeta) = the BatchNorm (+ activation) backward of BnReluUpF as a function of (dy, x, gamma).  With
+    up == 1 its backward is the double-backward kernel (the critics' gradient penalty); mean_invstd / scale_shift are
+    the forward's saved statistics, whose dependence on x and gamma is part of that kernel's formula.  The upsampling
+    form (up == 2, generator only) is first-order: differentiating it again raises."""
+
+    @staticmethod
+    def forward(ctx, dy, x, gamma, mean_invstd, scale_shift, relu, up):
+        dx, dgamma, dbeta = K.bn_backward(dy, x, mean_invstd, scale_shift, relu, up)
+        ctx.cfg = (relu, up)
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(dy, x, mean_invstd, scale_shift)
+        return dx, dgamma, dbeta
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, ggx, ggamma, ggbeta):
+        relu, up = ctx.cfg
+        if up != 1:
+            raise NotImplementedError("second-order graph through the upsampling BatchNorm backward")
+        dy, x, mean_invstd, scale_shift = ctx.saved_tensors
+        if ggx is None:
+            ggx = torch.zeros_like(x)
+        cont = lambda t: None if t is None else t.contiguous()
+        gx, gdy, dgamma = K.bn_backward_backward(dy, x, mean_invstd, scale_shift, ggx.contiguous(), cont(ggamma),
+                                                 cont(ggbeta), relu, 1)
+        return gdy, gx, dgamma, None, None, None, None
 
 
 def bn_relu_up(x, bn, relu=True, up=1):
