@@ -446,6 +446,14 @@ int t2v_rel_loss_bwd(int32_t count, const float* const* host_a, const float* con
 /* x_hat[b] = alpha[b] * real[b] + (1 - alpha[b]) * fake[b]  (gan/losses.py:140-145), fp32 (B, S)                 */
 int t2v_lerp_rows(const float* real, const float* fake, const float* alpha, float* out, int64_t B, int64_t S,
                   void* stream);
+/* Non-zero-centred penalty of a single-scale critic (gan/losses.py:180-186, combine = mean) on g fp32 (B, S), 16-byte
+ * aligned: norms[b] = ||g_b||_2, out = mean_b (norms[b] - 1)^2, reduced in a fixed order (bit-identical across calls).
+ * partials: caller-provided fp32 scratch of B * splits (splits >= 1: blocks per sample).  bwd: dg = gout * 2 (n_b - 1)
+ * / (n_b B) * g, 0 on rows with n_b = 0; gout on the device.  T2V_ERR_ARG for B < 1 or S % 4 != 0.             */
+int t2v_gp_norm_fwd(const float* g, float* partials, float* norms, float* out, int64_t B, int64_t S, int32_t splits,
+                    void* stream);
+int t2v_gp_norm_bwd(const float* g, const float* norms, const float* gout, float* dg, int64_t B, int64_t S,
+                    void* stream);
 
 /* Caption encoder / decoder recurrence (models/txt/basic.py:18-19,49-101: nn.Embedding + nn.LSTM on a
  * PackedSequence), replacing cuDNN.  gx fp32 [B][L][ndir][4H] = W_ih x + b_ih + b_hh (one GEMM on the engine);

@@ -163,6 +163,8 @@ SIGNATURES.update({
     "t2v_rel_loss_fwd": [c_i32, _PP, _PP, _I32P, _F32P, c_i32, _P, _P],
     "t2v_rel_loss_bwd": [c_i32, _PP, _PP, _PP, _PP, _I32P, _F32P, c_i32, _P, _P],
     "t2v_lerp_rows": [_P, _P, _P, _P, c_i64, c_i64, _P],
+    "t2v_gp_norm_fwd": [_P, _P, _P, _P, c_i64, c_i64, c_i32, _P],
+    "t2v_gp_norm_bwd": [_P, _P, _P, _P, c_i64, c_i64, _P],
     "t2v_lstm_pack_whh": [_P, _P, c_i32, c_i32, _P],
     "t2v_lstm_seq_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_i32, c_i32, c_i32, c_i32, _P],
     "t2v_lstm_seq_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_i32, c_i32, c_i32, c_i32, _P],

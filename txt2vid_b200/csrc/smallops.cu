@@ -7,8 +7,8 @@
 //     data / weight gradients (closed under the second differentiation of the penalty);
 //   * relativistic / Wasserstein loss reduction over all pyramid levels and prediction pairs in ONE launch forward and
 //     ONE backward (gan/losses.py:55-85, gan/cond_gan.py:51-61);
-//   * gradient-penalty arithmetic: per-sample interpolation (gan/losses.py:140-145) and the fp32 dot / scale kernels
-//     behind sum ||g||^2 and its derivative (losses.py:180-186).
+//   * gradient-penalty arithmetic: per-sample interpolation (gan/losses.py:140-145), the fp32 dot / scale kernels
+//     behind sum ||g||^2 and its derivative, and mean_b (||g_b|| - 1)^2 with its derivative (losses.py:180-186).
 #include "t2v_common.cuh"
 
 namespace t2v {
@@ -298,6 +298,76 @@ __global__ void lerp_rows_kernel(const float* __restrict__ real, const float* __
   out[i] = a * real[i] + (1.f - a) * fake[i];
 }
 
+// Non-zero-centred penalty mean_b (||g_b||_2 - 1)^2 of g (B, S) (gan/losses.py:180-186, combine = torch.mean).
+// Pass 1: block (sample b, split k) sums the squares of its contiguous chunk of row b with 16-byte loads into
+// partials[b * splits + k].  Which thread reads which element and the in-block tree depend on S and splits only,
+// so two calls give bit-identical sums (the fp32 mode relies on it, DESIGN §2).
+__global__ void __launch_bounds__(256) gp_norm_partial_kernel(const float* __restrict__ g, float* __restrict__ partials,
+                                                              long long S4, long long chunk4, int splits) {
+  __shared__ float red[8];
+  const long long blk = blockIdx.x;
+  const long long b = blk / splits;
+  const long long lo = (blk % splits) * chunk4, hi = min(S4, lo + chunk4);
+  const float4* row = reinterpret_cast<const float4*>(g) + b * S4;
+  float acc = 0.f;
+#pragma unroll 8
+  for (long long i = lo + threadIdx.x; i < hi; i += 256) {
+    const float4 v = __ldg(row + i);
+    acc = fmaf(v.x, v.x, acc);
+    acc = fmaf(v.y, v.y, acc);
+    acc = fmaf(v.z, v.z, acc);
+    acc = fmaf(v.w, v.w, acc);
+  }
+  acc = warp_sum(acc);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float t = 0.f;
+    for (int w = 0; w < 8; ++w) t += red[w];
+    partials[blk] = t;
+  }
+}
+// Pass 2 (one block): n_b = sqrt(sum of row b's partials, in split order); out = mean_b (n_b - 1)^2 over a fixed tree.
+__global__ void __launch_bounds__(256) gp_norm_finish_kernel(const float* __restrict__ partials, float* __restrict__ norms,
+                                                             float* __restrict__ out, long long B, int splits) {
+  __shared__ float red[8];
+  float acc = 0.f;
+  for (long long b = threadIdx.x; b < B; b += 256) {
+    const float* p = partials + b * splits;
+    float s = 0.f;
+    for (int k = 0; k < splits; ++k) s += p[k];
+    const float n = sqrtf(s);
+    norms[b] = n;
+    const float d = n - 1.f;
+    acc = fmaf(d, d, acc);
+  }
+  acc = warp_sum(acc);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float t = 0.f;
+    for (int w = 0; w < 8; ++w) t += red[w];
+    out[0] = t / (float)B;
+  }
+}
+// dg[b, s] = gout * 2 (n_b - 1) / (n_b B) * g[b, s]; 0 on a row with n_b = 0 (the subgradient torch's norm takes)
+__global__ void gp_norm_bwd_kernel(const float* __restrict__ g, const float* __restrict__ norms,
+                                   const float* __restrict__ gout, float* __restrict__ dg, long long S4,
+                                   long long total4, float B) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total4) return;
+  const float n = norms[i / S4];
+  const float c = n > 0.f ? gout[0] * (2.f * (n - 1.f) / (n * B)) : 0.f;
+  float4 v = __ldg(reinterpret_cast<const float4*>(g) + i);
+  v.x *= c;
+  v.y *= c;
+  v.z *= c;
+  v.w *= c;
+  reinterpret_cast<float4*>(dg)[i] = v;
+}
+
+static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
 }  // namespace t2v
 
 using namespace t2v;
@@ -439,6 +509,26 @@ int t2v_lerp_rows(const float* real, const float* fake, const float* alpha, floa
   lerp_rows_kernel<<<nblocks(total, 256), 256, 0, STREAM>>>(real, fake, alpha, out, S, total);
   count_launch();
   return check_last("lerp_rows");
+}
+
+int t2v_gp_norm_fwd(const float* g, float* partials, float* norms, float* out, int64_t B, int64_t S, int32_t splits,
+                    void* stream) {
+  if (B < 1 || S < 4 || S % 4 || splits < 1 || B * splits > 0x7fffffffLL) return T2V_ERR_ARG;
+  if (!g || !partials || !norms || !out || !aligned16(g)) return T2V_ERR_ARG;
+  const long long S4 = S / 4, chunk4 = (S4 + splits - 1) / splits;
+  gp_norm_partial_kernel<<<(unsigned)(B * splits), 256, 0, STREAM>>>(g, partials, S4, chunk4, splits);
+  gp_norm_finish_kernel<<<1, 256, 0, STREAM>>>(partials, norms, out, B, splits);
+  count_launch(2);
+  return check_last("gp_norm_fwd");
+}
+int t2v_gp_norm_bwd(const float* g, const float* norms, const float* gout, float* dg, int64_t B, int64_t S,
+                    void* stream) {
+  if (B < 1 || S < 4 || S % 4) return T2V_ERR_ARG;
+  if (!g || !norms || !gout || !dg || !aligned16(g) || !aligned16(dg)) return T2V_ERR_ARG;
+  const long long total4 = B * (S / 4);
+  gp_norm_bwd_kernel<<<nblocks(total4, 256), 256, 0, STREAM>>>(g, norms, gout, dg, S / 4, total4, (float)B);
+  count_launch();
+  return check_last("gp_norm_bwd");
 }
 
 }  // extern "C"

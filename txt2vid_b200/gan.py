@@ -168,6 +168,10 @@ def _gradient_penalty(discrim, real_x=None, real_xbar=None, fake_x=None, fake_xb
                             create_graph=True, retain_graph=True, only_inputs=True)[0]
     if zero_center and combine is torch.sum and g.numel() % 8 == 0:
         return ops.DotF.apply(g.contiguous(), g.contiguous())        # sum_b ||g_b||^2, one reduction kernel
+    # mean_b (||g_b|| - 1)^2 on the penalty kernels; ops.K lacks them only where tests put ops on a CPU spec
+    if not zero_center and combine is torch.mean and g.dtype == torch.float32 and (g.numel() // B) % 4 == 0 \
+            and hasattr(ops.K, "gp_norm_fwd"):
+        return ops.GradNormPenaltyF.apply(g.contiguous())
     n2 = g.reshape(B, -1).pow(2).sum(dim=1)
     return combine(n2) if zero_center else combine((n2.sqrt() - 1) ** 2)
 
@@ -232,9 +236,34 @@ class CondGan(object):
     def _mean_over_levels(loss, fakes, reals, idx):
         return torch.stack([loss(fake=f[idx], real=r[idx]) for f, r in zip(fakes, reals)]).mean()
 
+    @staticmethod
+    def _check_single_scale(discrim, cond, mapping):
+        if cond is not None:
+            raise ValueError("conditional single-scale critics (TCWYT) are not supported: %s was given captions"
+                             % type(discrim).__name__)
+        if mapping is not None:
+            raise ValueError("single-scale critics with a sample mapping (TCWYT's FrameMap) are not supported")
+
+    def _single_scale_forward(self, discrim, real, fake, loss, gp_lambda):
+        """A critic without `sub_discrims` (TGAN's VideoDiscrim: one scalar per call) on the one-level lists
+        multiscale_data gives.  D(real) runs before D(fake), as in the reference's discrim_forward: the BatchNorm
+        running statistics see the calls in that order.  The penalty is the non-zero-centred mean of
+        gan/losses.py:135-186."""
+        real_pred = discrim(x=real[0]) if real is not None else None
+        fake_pred = discrim(x=fake[0]) if fake is not None else None
+        l = None
+        if loss is not None and real_pred is not None and fake_pred is not None:
+            l = loss(fake=fake_pred, real=real_pred)
+            if gp_lambda > 0:
+                l = l + gp_lambda * _gradient_penalty(discrim, real_x=real[0], fake_x=fake[0])
+        return l, fake_pred, real_pred
+
     def discrim_forward(self, name=None, discrim=None, real=None, real_mapping=None, fake=None, fake_mapping=None,
                         real_cond=None, fake_cond=None, loss=None, gp_lambda=-1):
         """(x_r,c_r) / (x_r,c_f) / (x_f,c_r) pairs and their per-level loss average (cond_gan.py:34-87)."""
+        if not hasattr(discrim, "sub_discrims"):
+            self._check_single_scale(discrim, real_cond, real_mapping if real_mapping is not None else fake_mapping)
+            return self._single_scale_forward(discrim, real, fake, loss, gp_lambda)
         fake_pred = real_pred = l = None
         if real_cond is not None and fake_cond is not None:
             pair = loss is not None and hasattr(discrim, "forward_pair") and real_mapping is None \
@@ -293,6 +322,10 @@ class CondGan(object):
         fake_mapping = self._map_input(fake)
         losses = []
         for r, name, discrim in zip(real_pred, self.discrim_names, self.discrims):
+            if not hasattr(discrim, "sub_discrims"):
+                self._check_single_scale(discrim, cond, fake_mapping)
+                losses.append(loss(fake=discrim(x=fake[0]), real=r))
+                continue
             fake_cc = discrim(x=fake, cond=cond, xbar=fake_mapping)
             mode = fused_loss_mode(loss, "g")
             pick = lambda t: t[0] if isinstance(t, (tuple, list)) else t

@@ -1305,6 +1305,33 @@ def lerp_rows(real, fake, alpha):
     return out
 
 
+def gp_norm_fwd(g):
+    """g fp32 (B, ...) -> (0-d mean_b (||g_b|| - 1)^2, norms fp32 (B,)), reduced in a fixed order.  One block per
+    8192 elements of a row (at most 1024 per row): enough blocks to fill the GPU at B = 1."""
+    require_cuda(g)
+    assert g.dtype == F32 and g.is_contiguous()
+    B = g.shape[0]
+    S = g.numel() // max(B, 1)
+    splits = max(1, min(1024, -(-S // 8192)))
+    partials = torch.empty(B * splits, device=g.device, dtype=F32)
+    norms = torch.empty(B, device=g.device, dtype=F32)
+    out = torch.empty((), device=g.device, dtype=F32)
+    check(lib().t2v_gp_norm_fwd(ptr(g), ptr(partials), ptr(norms), ptr(out), B, S, splits, stream()),
+          "t2v_gp_norm_fwd")
+    return out, norms
+
+
+def gp_norm_bwd(g, norms, gout):
+    """d/dg of gp_norm_fwd's penalty times gout (0-d fp32 on the device)"""
+    require_cuda(g, norms, gout)
+    assert g.dtype == F32 and g.is_contiguous() and norms.dtype == F32 and gout.dtype == F32 and gout.numel() == 1
+    B = g.shape[0]
+    dg = torch.empty_like(g)
+    check(lib().t2v_gp_norm_bwd(ptr(g), ptr(norms), ptr(gout), ptr(dg), B, g.numel() // max(B, 1), stream()),
+          "t2v_gp_norm_bwd")
+    return dg
+
+
 # ------------------------------------------------------------------------------------- caption LSTM
 def lstm_pack_whh(whh):
     """fp32 (ndir, 4H, H) -> (ndir, H, 4H)"""

@@ -1323,6 +1323,23 @@ class DotF(Function):
         return da, db
 
 
+class GradNormPenaltyF(Function):
+    """0-d fp32 mean_b (||g_b||_2 - 1)^2 of g fp32 (B, ...): the non-zero-centred gradient penalty (gan/losses.py:
+    180-186).  Its backward feeds the double backward through the critic; nothing differentiates it again."""
+
+    @staticmethod
+    def forward(ctx, g):
+        out, norms = K.gp_norm_fwd(g)
+        ctx.save_for_backward(g, norms)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gout):
+        g, norms = ctx.saved_tensors
+        return K.gp_norm_bwd(g, norms, gout.contiguous().reshape(()).float())
+
+
 class ScaleAddF(Function):
     """y = s * o + x: the non-local block's output gamma * o + x (models/layers.py:36,68); s None: y = o + x"""
 

@@ -99,7 +99,7 @@ def test(gan=None, num_samples=1, dataset=None, device=None, params=None, channe
                 _, _, cond = gan.cond_encoder.encode(y[0], y[1])
             z = torch.randn(B, gan.gen.latent_size, device=device)
             with torch.no_grad():
-                fake = gan(z, cond=cond)
+                fake = as_levels(gan(z, cond=cond))
             save_frames(x, path='%s/real_%d.png' % (params.out_samples, i), channel_first=channel_first,
                         is_images=params.img_model)
             if cond is not None:
@@ -110,6 +110,11 @@ def test(gan=None, num_samples=1, dataset=None, device=None, params=None, channe
                 status("saving to %s" % path)
                 save_frames(f, path=path, channel_first=channel_first, is_images=params.img_model)
             break
+
+
+def as_levels(fake):
+    """generator output as a list of pyramid levels: a single-scale generator (TGAN) returns one tensor"""
+    return [fake] if torch.is_tensor(fake) else fake
 
 
 def encode_captions(gan, y, end2end):
@@ -132,7 +137,7 @@ def _d_phase(gan, x, cond, device, params, losses, z, channel_first, end2end, j=
         xs, conds = multiscale_data(x, cond, params.frame_sizes, params.subsample_input)
         if z is None:
             z = torch.randn(B, gan.gen.latent_size, device=device)
-        fake = gan(z, cond=conds[0] if conds is not None else None)
+        fake = as_levels(gan(z, cond=conds[0] if conds is not None else None))
         st = {"xs": xs, "conds": conds, "z": z, "fake": fake}
     loss = gan.discrim_step(real=st["xs"], fake=[f.detach() for f in st["fake"]], cond=st["conds"],
                             loss=losses.discrim_loss, gp_lambda=params.gp_lambda)
@@ -162,7 +167,7 @@ def _g_phase(gan, st, params, losses, j=0, end2end=False):
             with torch.enable_grad() if need_graph else torch.no_grad():
                 _, _, st["real_pred"] = gan.all_discrim_forward(real=xs, cond=conds, fake=None, loss=None)
         else:
-            st["fake"] = gan(st["z"], cond=conds[0] if conds is not None else None)
+            st["fake"] = as_levels(gan(st["z"], cond=conds[0] if conds is not None else None))
         loss = gan.gen_step(fake=st["fake"], real_pred=st["real_pred"], cond=conds, loss=losses.gen_loss)
         if not params.no_mean_gen_loss:
             loss = loss / params.gen_steps
@@ -211,11 +216,13 @@ class GraphedTrainStep(object):
     Everything the host decides per iteration reaches the kernels through device buffers refreshed before each replay: the batch, the caption
     embedding (the Bi-LSTM runs eagerly -- variable lengths), the host-RNG draws (hostrng.StaticDraws, same
     generators and order as the reference), Adam's bias corrections.  z comes from the CUDA generator inside
-    the graph.  Needs discrim_steps = gen_steps = 1, a fixed batch shape and an even frame count per level."""
+    the graph.  With discrim_steps > 1 (the WGAN-GP recipe: 5 critic steps per generator step) the graph holds every
+    critic step, each with its all-reduce and Adam step; each of those Adam steps reads its own row of bias corrections.
+    Needs gen_steps = 1, a fixed batch shape and an even frame count per level."""
 
     def __init__(self, gan, optD, optG, params, losses, device, channel_first=True, end2end=False, dist=None,
                  warmup=2):
-        assert params.discrim_steps == 1 and params.gen_steps == 1 and not end2end
+        assert params.gen_steps == 1 and not end2end
         self.gan, self.optD, self.optG, self.params, self.losses = gan, optD, optG, params, losses
         self.device, self.channel_first, self.dist = device, channel_first, dist
         self.warmup, self.calls, self.graphs = warmup, 0, None
@@ -229,10 +236,12 @@ class GraphedTrainStep(object):
 
     # ---- per-replay host work
     def _stage_adam(self, opt, step, slot):
+        """row j of opt.dyn <- the bias corrections of Adam step `step + j` (one row per captured step)"""
         b1, b2 = opt.param_groups[0]["betas"]
+        lr = opt.param_groups[0]["lr"]
         h = opt._dyn_host[slot]
-        h[0] = opt.param_groups[0]["lr"] / (1.0 - b1 ** step)
-        h[1] = 1.0 / (1.0 - b2 ** step) ** 0.5
+        h.copy_(torch.tensor([[lr / (1.0 - b1 ** t), 1.0 / (1.0 - b2 ** t) ** 0.5]
+                              for t in range(step, step + h.shape[0])], dtype=torch.float32))
         K.multi_copy([h], [opt.dyn])            # UVA read of the pinned slot (see hostrng.StaticDraws.refresh)
 
     def _capture(self, x, cond):
@@ -240,9 +249,9 @@ class GraphedTrainStep(object):
         dev = self.device
         self.static_x = x.clone()
         self.static_cond = None if cond is None else cond.clone()
-        for opt in (self.optD, self.optG):
-            opt.dyn = torch.zeros(2, device=dev, dtype=torch.float32)
-            opt._dyn_host = [torch.zeros(2, dtype=torch.float32).pin_memory() for _ in range(self.ring)]
+        for opt, n in ((self.optD, self.params.discrim_steps), (self.optG, 1)):
+            opt.dyn = torch.zeros(n, 2, device=dev, dtype=torch.float32)
+            opt._dyn_host = [torch.zeros(n, 2, dtype=torch.float32).pin_memory() for _ in range(self.ring)]
             opt._step_count = max([st_["step"] for st_ in opt.state.values()] or [0])
             opt.zero_grad(set_to_none=True)
         torch.cuda.synchronize()
@@ -253,12 +262,20 @@ class GraphedTrainStep(object):
         # between them leave cross-stream waits in front of each replay: measured at two GPUs the step then
         # flips between 90 and 130 ms.
         g = torch.cuda.CUDAGraph()
+        dynD = self.optD.dyn
         with torch.cuda.graph(g, pool=pool, stream=self.side, capture_error_mode="thread_local"):
-            st = _d_phase(self.gan, self.static_x, self.static_cond, dev, self.params, self.losses, None,
-                          self.channel_first, False)
-            if self.dist is not None:
-                self.dist.reduce_grads(self.optD)
-            self.optD.step()
+            st = None
+            for j in range(self.params.discrim_steps):
+                st = _d_phase(self.gan, self.static_x, self.static_cond, dev, self.params, self.losses, None,
+                              self.channel_first, False, j, st)
+                if self.dist is not None:
+                    self.dist.reduce_grads(self.optD)
+                self.optD.dyn = dynD[j]
+                self.optD.step()
+                # the iteration's lossD is the sum over its critic steps, as train_iteration returns it
+                lossD = st["lossD"] if j == 0 else lossD + st["lossD"]
+            self.optD.dyn = dynD
+            st["lossD"] = lossD
             st = _g_phase(self.gan, st, self.params, self.losses)
             if self.dist is not None:
                 self.dist.reduce_grads(self.optG)
@@ -317,8 +334,8 @@ class GraphedTrainStep(object):
         self.stage_evt[slot] = torch.cuda.Event()
         self.stage_evt[slot].record()
         self.graphs[0].replay()
-        for opt in (self.optD, self.optG):
-            opt._step_count += 1
+        self.optD._step_count += self.params.discrim_steps
+        self.optG._step_count += 1
         ops.bump_weight_epoch()          # eager users of the modules must re-pack the updated weights
         return self.state["lossD"], self.state["lossG"]
 
@@ -406,7 +423,7 @@ def train(gan=None, num_epoch=None, dataset=None, device=None, optD=None, optG=N
     main_rank = dist is None or getattr(dist, "is_main", True)     # checkpoints / samples / logs: rank 0 only
     graphed = None
     if getattr(params, 'cuda_graphs', False) and torch.device(device).type == 'cuda' and not end2end \
-            and params.discrim_steps == 1 and params.gen_steps == 1:
+            and params.gen_steps == 1:
         graphed = GraphedTrainStep(gan, optD, optG, params, losses, torch.device(device), channel_first=channel_first,
                                    end2end=False, dist=dist)
     lagged = LaggedLosses(_log_losses, lag=2 if graphed is not None else 0, device=device)
