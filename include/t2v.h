@@ -35,9 +35,10 @@ extern "C" {
 /* algo selector for the convolution engine */
 #define T2V_ALGO_AUTO 0   /* tcgen05 implicit GEMM when the shape allows it, else SIMT */
 #define T2V_ALGO_TC 1     /* force the tcgen05/TMEM/TMA kernel (error if shape unsupported) */
-#define T2V_ALGO_SIMT 2   /* force the CUDA-core kernel (cross-check + odd shapes) */
+#define T2V_ALGO_SIMT 2   /* force the CUDA-core kernels of t2v_gconv_* (cross-check + odd shapes) */
 #define T2V_ALGO_TC_GENERIC 3 /* force the generic tcgen05 implicit GEMM (skip the halo-resident 64-channel kernels) */
-#define T2V_ALGO_SIMT_F32 4   /* t2v_conv_wgrad only: dy and x are fp32 CL, CUDA-core fp32 FMA (fp32 parity mode) */
+#define T2V_ALGO_SIMT_F32 4   /* t2v_conv_wgrad only: dy and x are fp32 CL, on the kernel of t2v_gconv_wgrad_f32:
+                               * exact fp32 FMAs (fp32 parity mode) */
 
 /* epilogue flags of t2v_conv_fprop */
 #define T2V_EPI_RELU 1u       /* y = max(y, 0) after bias/residual */
@@ -46,8 +47,9 @@ extern "C" {
                                * adding it, zero the output where r <= 0 -- the backward of the ReLU that produced the
                                * convolution's input, fused into the data-gradient epilogue (layers.py:230-232) */
 #define T2V_EPI_IN_F32 16u    /* fp32 PARITY mode: x / residual are fp32 CL and w is fp32 [Cout][taps][Cin]; the
-                               * convolution runs as exact fp32 FMAs on the CUDA cores (the reference's numerics; the
-                               * tensor pipe's truncating fp32 accumulator cannot reach 1e-6 on K ~ 1e4), y fp32 */
+                               * convolution runs on the kernel of t2v_gconv_fprop_f32 as exact fp32 FMAs, flushed
+                               * once per tap (the reference's numerics; the tensor pipe's truncating fp32 accumulator
+                               * cannot reach 1e-6 on K ~ 1e4), y fp32 */
 
 /* Stride-1, "same"-padded convolution geometry (every conv on the TGANv2 path:
  * models/layers.py:174,177,183,231,233,237,251; models/resnet3d.py:12-17; 1x1(x1) convs of the
@@ -341,9 +343,11 @@ int t2v_multi_copy(int32_t count, const float* const* host_src, float* const* ho
  * fp32 ACTIVATION STORAGE (the "fp32 parity mode": BASELINE north_star, 1e-3 relative on losses and gradients).
  * Every entry point above whose activations are bf16 CL has a twin with the suffix _f32 and the SAME signature
  * in which those tensors are fp32 CL (same kernels instantiated for float storage; arithmetic is fp32 in both).
- * Convolutions on fp32 storage bypass the bf16 tensor pipe and run as exact fp32 FMAs on the CUDA cores:
- * t2v_conv_fprop / t2v_conv_dgrad with T2V_EPI_IN_F32, t2v_conv_wgrad with T2V_ALGO_SIMT_F32, and the
- * t2v_gconv_*_f32 entry points below.                                                                          */
+ * Convolutions on fp32 storage bypass the bf16 tensor pipe and run as exact fp32 FMAs on the CUDA cores, all on the
+ * kernels of the t2v_gconv_*_f32 entry points below: an accumulator per tap (FMA chains of at most Cin terms) added
+ * into the total in ascending tap order, and in the weight gradient a flush every 1024 positions.
+ * t2v_conv_fprop / t2v_conv_dgrad with T2V_EPI_IN_F32 and t2v_conv_wgrad with T2V_ALGO_SIMT_F32 reach the same
+ * kernels for their stride-1 "same" geometry.                                                                  */
 int t2v_relu_fwd_f32(const void* x, void* y, int64_t n, void* stream);
 int t2v_relu_bwd_f32(const void* dy, const void* ref, void* dx, int64_t n, void* stream);
 int t2v_leaky_relu_fwd_f32(const void* x, void* y, int64_t n, float slope, void* stream);

@@ -306,6 +306,24 @@ def test_wgrad_small_channels_auto(case):
     assert _rel(dw, K.conv_wgrad(dy, x, k=k, algo=2)) < 2e-3          # CUDA-core cross-check
 
 
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32], ids=["bf16", "fp32"])
+def test_gconv_same_matches_cuda_core_conv(dtype, monkeypatch):
+    """A stride-1 "same" layer through t2v_gconv_fprop (bf16, engine routes off) or t2v_gconv_fprop_f32 and through the
+    CUDA-core route of t2v_conv_fprop (algo = 2, or the fp32 parity mode) is one kernel with one summation order
+    (16-channel chunks, one flush per tap): bit-identical outputs."""
+    from txt2vid_b200 import kernels as K
+    monkeypatch.setattr(K, "GCONV_TC", False)
+    N, D, H, W, Cin, Cout, k = 3, 3, 6, 10, 64, 80, (3, 3, 3)
+    g = torch.Generator(device="cuda").manual_seed(6)
+    x = torch.randn((N, D, H, W, Cin), device="cuda", generator=g).to(dtype)
+    w = (torch.randn((Cout, 27, Cin), device="cuda", generator=g) / (27 * Cin) ** 0.5).to(dtype)
+    bias = torch.randn(Cout, device="cuda", generator=g)
+    for out_f32 in (True, False) if dtype == torch.bfloat16 else (True,):
+        y = K.gconv_fprop(x, w, bias, k, (1, 1, 1), (1, 1, 1), out_f32=out_f32)
+        ref = K.conv_fprop(x, w, bias=bias, k=k, out_f32=out_f32, algo=2)
+        assert y.dtype == ref.dtype and torch.equal(y, ref)
+
+
 def test_simt_odd_channels():
     from txt2vid_b200 import kernels as K
     case = (4, 2, 4, 4, 3, 5, (3, 3, 3))

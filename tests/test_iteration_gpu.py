@@ -42,7 +42,7 @@ def _record(tag, payload):
                                                       ("tganv2_uncond_B8.json", False, False)])
 def test_full_iteration_fp32_mode_on_b200(name, conditional, perturb):
     """BASELINE north_star, fp32 bar: one full iteration through the REAL kernels in the fp32 storage mode (same
-    typed kernels instantiated for float, tcgen05 engine on bf16 hi/lo operand splits) within 1e-3 relative of the
+    typed kernels instantiated for float, convolutions as exact fp32 FMAs on the CUDA cores) within 1e-3 relative of the
     oracle on both losses, the generated clips and the gradients of G and D -- with the non-local blocks switched on
     (gamma = 0.5) and non-trivial BatchNorm affine parameters in the `perturb` case."""
     from test_product_vs_oracle_cpu import adam_update_stats

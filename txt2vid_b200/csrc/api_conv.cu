@@ -21,9 +21,9 @@ int halo_wgrad_launch(const t2v_conv_geom*, const void*, const void*, float*, in
 bool halo_sd2_supported(const t2v_conv_geom* g);
 int halo_fprop_sd2_launch(const t2v_conv_geom*, const void*, const void*, const float*, void*, uint32_t, cudaStream_t);
 int halo_dgrad_sd2_launch(const t2v_conv_geom*, const void*, const void*, const void*, void*, uint32_t, cudaStream_t);
-int simt_fprop_launch(const t2v_conv_geom*, const void*, const void*, const float*, const void*, void*,
-                      uint32_t, cudaStream_t);
-int simt_wgrad_launch(const t2v_conv_geom*, const void*, const void*, float*, int, cudaStream_t, int in_f32 = 0);
+int gconv_fprop_launch(const t2v_gconv_geom*, const void*, const void*, const float*, const void*, void*, uint32_t,
+                       bool f32, cudaStream_t);
+int gconv_wgrad_launch(const t2v_gconv_geom*, const void*, const void*, float*, int, bool f32, cudaStream_t);
 void prof_enable(int on);
 void prof_read(double* out, int nkinds);
 void prof_next_scale(double s);
@@ -105,6 +105,12 @@ __global__ void fold_pairs_kernel(const float* __restrict__ dw2, float* __restri
 
 using namespace t2v;
 
+// A stride-1 "same" convolution as a general geometry: the CUDA-core route of the t2v_conv_* entry points.
+static t2v_gconv_geom same_geom(const t2v_conv_geom* g) {
+  return t2v_gconv_geom{g->N, g->D, g->H, g->W, g->D, g->H, g->W, g->Cin, g->Cout,
+                        g->kd, g->kh, g->kw, 1, 1, 1, g->kd / 2, g->kh / 2, g->kw / 2};
+}
+
 extern "C" {
 
 int t2v_version(void) { return 100; }
@@ -119,15 +125,16 @@ int t2v_conv_fprop(const t2v_conv_geom* g, const void* x, const void* w, const f
                    const void* residual, void* y, uint32_t epi_flags, int algo, void* stream) {
   if (!g || !x || !w || !y) return T2V_ERR_ARG;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const t2v_gconv_geom gg = same_geom(g);
   if (epi_flags & T2V_EPI_IN_F32) {             // fp32 parity mode: fp32 operands on the CUDA-core FFMA kernel
     if (algo == T2V_ALGO_TC || algo == T2V_ALGO_TC_GENERIC) return T2V_ERR_ARG;
     if ((epi_flags & T2V_EPI_RELU_MASK) && !residual) return T2V_ERR_ARG;
-    return simt_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
+    return gconv_fprop_launch(&gg, x, w, bias, residual, y, epi_flags, true, s);
   }
   const bool tc_ok = igemm_fprop_supported(g);
   if ((algo == T2V_ALGO_TC || algo == T2V_ALGO_TC_GENERIC) && !tc_ok) return T2V_ERR_ARG;
   if ((epi_flags & T2V_EPI_RELU_MASK) && (algo == T2V_ALGO_SIMT || !tc_ok || !residual)) return T2V_ERR_ARG;
-  if (algo == T2V_ALGO_SIMT || !tc_ok) return simt_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
+  if (algo == T2V_ALGO_SIMT || !tc_ok) return gconv_fprop_launch(&gg, x, w, bias, residual, y, epi_flags, false, s);
   if (algo != T2V_ALGO_TC_GENERIC && halo_fprop_supported(g)) return halo_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
   return igemm_fprop_launch(g, x, w, bias, residual, y, epi_flags, s);
 }
@@ -145,10 +152,11 @@ int t2v_conv_wgrad(const t2v_conv_geom* g, const void* dy, const void* x, float*
                    int algo, void* stream) {
   if (!g || !dy || !x || !dw) return T2V_ERR_ARG;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  if (algo == T2V_ALGO_SIMT_F32) return simt_wgrad_launch(g, dy, x, dw, accumulate, s, 1);   // fp32 dy / x
+  const t2v_gconv_geom gg = same_geom(g);
+  if (algo == T2V_ALGO_SIMT_F32) return gconv_wgrad_launch(&gg, dy, x, dw, accumulate, true, s);   // fp32 dy / x
   const bool tc_ok = igemm_wgrad_supported(g);
   if ((algo == T2V_ALGO_TC || algo == T2V_ALGO_TC_GENERIC) && !tc_ok) return T2V_ERR_ARG;
-  if (algo == T2V_ALGO_SIMT || !tc_ok) return simt_wgrad_launch(g, dy, x, dw, accumulate, s);
+  if (algo == T2V_ALGO_SIMT || !tc_ok) return gconv_wgrad_launch(&gg, dy, x, dw, accumulate, false, s);
   if (algo != T2V_ALGO_TC_GENERIC && halo_wgrad_supported(g)) return halo_wgrad_launch(g, dy, x, dw, accumulate, s, 0);
   return igemm_wgrad_launch(g, dy, x, dw, accumulate, s);
 }

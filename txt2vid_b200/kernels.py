@@ -48,11 +48,12 @@ def _act(*ts):
         assert t is None or (t.dtype in (BF16, F32) and t.is_contiguous()), (None if t is None else (t.dtype, t.shape))
 
 
-# fp32 storage mode, convolution engine: fp32 operands, exact fp32 FMAs on the CUDA cores (simt_conv.cu,
-# T2V_EPI_IN_F32): the reference's own numerics, ~1e-6 per layer -- what the 1e-3 bar on GRADIENTS needs on this
-# network (a forward deviation of 5e-5 already moves the generator's gradients by 5e-3 through ReLU / BatchNorm,
-# measured).  The tensor pipe on bf16 part splits of the fp32 operands does not reach it: its fp32 accumulator
-# truncates on every MMA (7e-6 relative at K = 1024, 3e-5 at K = 9216; profiles/r02_fp32_engine_accuracy.txt).
+# fp32 storage mode, convolution engine: fp32 operands, exact fp32 FMAs on the CUDA cores (gconv.cu, selected by
+# T2V_EPI_IN_F32 / T2V_ALGO_SIMT_F32): the reference's own numerics, ~1e-6 per layer -- what the 1e-3 bar on
+# GRADIENTS needs on this network (a forward deviation of 5e-5 already moves the generator's gradients by 5e-3 through
+# ReLU / BatchNorm, measured).  The tensor pipe on bf16 part splits of the fp32 operands does not reach it: its fp32
+# accumulator truncates on every MMA (7e-6 relative at K = 1024, 3e-5 at K = 9216;
+# profiles/r02_fp32_engine_accuracy.txt).
 
 
 def _geom(N, D, H, W, Cin, Cout, k):
@@ -159,20 +160,10 @@ def conv_dgrad(dy, wT, k=(3, 3, 3), residual=None, relu=False, out_f32=False, al
 def conv_wgrad(dy, x, k=(3, 3, 3), out=None, accumulate=False, algo=0):
     """dw (Cout,taps,Cin) fp32 = sum_pos dy[pos,co] x[pos+tap,ci]."""
     require_cuda(dy, x)
-    if dy.dtype == F32:
-        assert x.dtype == F32 and dy.is_contiguous() and x.is_contiguous() and x.shape[:4] == dy.shape[:4]
-        N, D, H, W, Cout = dy.shape
-        Cin = x.shape[-1]
-        taps = k[0] * k[1] * k[2]
-        if out is None:
-            assert not accumulate
-            out = torch.empty((Cout, taps, Cin), device=x.device, dtype=F32)
-        g = _geom(N, D, H, W, Cin, Cout, k)
-        check(lib().t2v_conv_wgrad(ctypes.byref(g), ptr(dy), ptr(x), ptr(out), 1 if accumulate else 0,
-                                   _lib.ALGO_SIMT_F32, stream()), "t2v_conv_wgrad")
-        return out
     N, D, H, W, Cout = dy.shape
     Cin = x.shape[-1]
+    if dy.dtype == F32:                           # fp32 parity mode on exact fp32 FMAs
+        algo = _lib.ALGO_SIMT_F32
     if (algo == 0 and tuple(k) == (1, 3, 3) and D == 1 and Cin == 32 and Cout in (16, 32)
             and W % 2 == 0 and W >= 16 and H >= 4 and dy.is_contiguous() and x.is_contiguous()):
         # 32-channel rows are 64 bytes: TMA and the MMA tiles run half empty.  Pair adjacent w voxels (a free view):
@@ -185,7 +176,7 @@ def conv_wgrad(dy, x, k=(3, 3, 3), out=None, accumulate=False, algo=0):
               "t2v_wgrad_fold_pairs")
         return out
     assert x.shape[:4] == dy.shape[:4] and dy.is_contiguous() and x.is_contiguous()
-    assert dy.dtype == BF16 and x.dtype == BF16
+    assert x.dtype == dy.dtype and dy.dtype in (BF16, F32)
     taps = k[0] * k[1] * k[2]
     if out is None:
         assert not accumulate

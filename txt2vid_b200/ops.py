@@ -36,10 +36,10 @@ def round16(c):
 # ------------------------------------------------------------------------------------- precision mode
 # "bf16": the product (bf16 activation storage, bf16 tensor-core operands, fp32 accumulation / statistics / master
 #         weights) -- BASELINE north_star's 2e-2 bar;
-# "fp32": fp32 activation storage on the same kernels instantiated for float, the tcgen05 engine fed with bf16 hi / lo
-#         operand splits (16 mantissa bits per operand, fp32 accumulation) -- the 1e-3 bar.  The bf16-only fusions
-#         (direct RGB stem, stride-(2,1,1) stem conv, fused skip conv, fused generator attention) fall back to their
-#         unfused formulations on the generic kernels.
+# "fp32": fp32 activation storage on the same kernels instantiated for float, every convolution as exact fp32 FMAs on
+#         the CUDA-core kernels of gconv.cu (fp32 accumulation flushed once per tap) -- the 1e-3 bar.  The bf16-only
+#         fusions (direct RGB stem, stride-(2,1,1) stem conv, fused skip conv, fused generator attention) fall back to
+#         their unfused formulations on the generic kernels.
 PRECISION = ["bf16"]
 
 
